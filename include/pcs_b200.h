@@ -206,6 +206,15 @@ PCS_API int pcs_p2p_status(pcs_problem* p, int* timed_out);
 
 /* Levenberg-Marquardt on the device (replaces scipy.optimize.least_squares TRF + LSMR as driven by
  * run_bundle_adjustment, optimisation_handling.py:52-117). */
+/* Termination, tested in this order in every iteration, after the damped step dx has been solved at the current
+ * linearisation point x (x, dx and g = J^T r range over the FREE parameters only; fixed entries of the parameter string
+ * do not enter any norm):
+ *   gtol  |g|_inf < gtol                          status 1, x is returned (the step is not taken);
+ *   xtol  |dx|_2 < xtol (xtol + |x|_2)            status 3, x is returned (the step is not taken);
+ *   ftol  after an ACCEPTED step, (c - c') / c < ftol with c, c' = r.r before / after the step: status 2, x + dx returned.
+ * A step is accepted when rho = (c - c') / pred > 0, pred = dx . (lambda D dx - g), D = diag(J^T J); then
+ * lambda <- max(lambda_min, lambda max(1/3, 1 - (2 rho - 1)^3)), nu = 2; otherwise lambda <- min(lambda_max, lambda nu),
+ * nu <- 2 nu, and reaching lambda_max ends the solve with status -1.  max_iter counts accepted and rejected steps. */
 typedef struct pcs_lm_options {
     int32_t max_iter;      /* default 100 (the reference's max_nfev, template_handler.py:24-31) */
     int32_t verbose;

@@ -548,12 +548,12 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
     double pred = 0.0, dx2 = 0.0, x2 = 0.0, ginf = 0.0;
     if (t < total) {
         double d, D, g;
-        bool replicated;
+        bool replicated, f;
         if (t < n_cam) {
             int c, a;
             if (t < 9 * (int64_t)C) { c = (int)(t / 9); a = (int)(t % 9); }
             else { c = (int)((t - 9 * (int64_t)C) / 6); a = 9 + (int)((t - 9 * (int64_t)C) % 6); }
-            const bool f = cam_mask[c] & (1u << a);
+            f = cam_mask[c] & (1u << a);
             d = f ? dc[c * 15 + a] : 0.0;
             D = f ? U[c * 225 + a * 16] : 0.0;
             g = f ? gc[c * 15 + a] : 0.0;
@@ -561,7 +561,7 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
         } else if (t < n_cam + n_pose) {
             const int64_t r = t - n_cam;
             const int m = (int)(r / 6), a = (int)(r % 6);
-            const bool f = pose_mask[m] & (1u << a);
+            f = pose_mask[m] & (1u << a);
             d = f ? dp[r] : 0.0;
             D = f ? V[(int64_t)m * 36 + a * 7] : 0.0;
             g = f ? gp[r] : 0.0;
@@ -569,7 +569,7 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
         } else {
             const int64_t j = t - n_cam - n_pose;
             const int k = (int)(j / 3), a = (int)(j % 3);
-            const bool f = key_mask[k] & (1u << a);
+            f = key_mask[k] & (1u << a);
             d = f ? dc[n_cam + j] : 0.0;
             D = f ? Pk[(int64_t)k * 9 + a * 4] : 0.0;
             g = f ? gk[j] : 0.0;
@@ -580,7 +580,7 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
         pred = d * (lambda * D * d - g);
         if (!replicated || rank0) {
             dx2 = d * d;
-            x2 = params[t] * params[t];
+            x2 = f ? params[t] * params[t] : 0.0;   // |x| of the xtol test is the norm of the FREE vector
         }
         if (!replicated) ginf = fabs(g);  // the replicated gradient norm is taken from the all-reduced copy (k_lm_take_step)
     }
