@@ -196,7 +196,7 @@ PCS_API int pcs_gauge_scale(int device, int64_t n_points, const double* estimate
  * problem's stream) -- the caller must put a barrier across the ranks between the setup call and the first exchange.
  * pcs_p2p_allreduce_camera_blocks enqueues one kernel (one CTA per peer) on the problem's stream: the rank's block is
  * pushed into its slot at every peer without fence or flag, the arrival of the data is the signal (csrc/pcs_p2p.cu);
- * all ranks must call it the same number of times.  PCS_P2P_SENTINEL=0 selects the older fence + flag protocol.
+ * all ranks must call it the same number of times.
  * pcs_p2p_status: *timed_out = 1 if a poll ever gave up waiting for a peer (the sums of that exchange are then
  * invalid); synchronises the stream.  No reference counterpart (the reference is single-process). */
 PCS_API int64_t pcs_p2p_buffer_bytes(const pcs_problem* p, int world_size);
@@ -267,7 +267,7 @@ PCS_API int pcs_timing_get(pcs_problem* p, double* normal_kernel_ms);
 PCS_API int pcs_timing_get_all(pcs_problem* p, double* ms, int64_t capacity, int64_t* n_out);
 
 /* Number of kernels of this library launched so far for the residual / Jacobian / normal-equation evaluations of
- * this problem (cuBLAS / cuSOLVER launches inside pcs_lm_solve are not counted).  bench.py reports the difference
+ * this problem (cuSOLVER launches inside pcs_lm_solve are not counted).  bench.py reports the difference
  * over its timed region as `gpu_launches`. */
 PCS_API int pcs_launch_count(const pcs_problem* p, int64_t* n_kernels);
 

@@ -39,7 +39,6 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
     if not force and not needs_build():
         return LIB
     nvcc = _nvcc()
-    extra = ["-DPCS_NE_KNOCKOUT"] if os.environ.get("PCS_BUILD_KNOCKOUT") == "1" else []   # tools/kne_knockout.sh only
     objdir = PKG / "build"
     objdir.mkdir(exist_ok=True)
     procs, objs = [], []
@@ -49,7 +48,7 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
             continue
         obj = objdir / (src.stem + ".o")
         objs.append(str(obj))
-        cmd = [nvcc, *NVCC_FLAGS, *extra, "-c", str(src), "-o", str(obj)]
+        cmd = [nvcc, *NVCC_FLAGS, "-c", str(src), "-o", str(obj)]
         if verbose:
             cmd[1:1] = ["-Xptxas", "-v"]
         procs.append((cmd, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
@@ -60,7 +59,7 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
         if pr.returncode != 0:
             raise RuntimeError("nvcc failed: " + " ".join(cmd) + "\n" + (out or ""))
     link = [nvcc, "-shared", "-o", str(LIB), *objs, "-gencode", "arch=compute_100a,code=sm_100a",
-            "-cudart", "static", "-lcublas", "-lcusolver", "-Xlinker", "--no-undefined"]
+            "-cudart", "static", "-lcusolver", "-Xlinker", "--no-undefined"]
     subprocess.check_call(link)
     return LIB
 

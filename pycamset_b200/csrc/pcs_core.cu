@@ -283,10 +283,9 @@ int launch_cost_only(pcs_problem* p, double* cost_dev)
 // row pair in registers; a warp's rows are contiguous in the CSR value array, so they are compacted
 // (fixed columns dropped) into shared memory and leave the SM as ONE bulk asynchronous copy
 // (cp.async.bulk shared -> global, the TMA unit): the copy-out does not pass through the load / store
-// unit, which is what bounds this kernel (BULK = false keeps the coalesced 8-byte load + store loop
-// for A/B runs: PCS_JAC_BULK=0).  28 B in + 16 P B out per observation.
+// unit, which is what bounds this kernel.  28 B in + 16 P B out per observation.
 // ------------------------------------------------------------------------------------------------
-template <int P, bool BULK>
+template <int P>
 __global__ void __launch_bounds__(128)
 k_jacobian(int64_t N, const int32_t* __restrict__ cam, const int32_t* __restrict__ pose, const int32_t* __restrict__ key,
            const double2* __restrict__ uv, const double* __restrict__ camtab, const double* __restrict__ posetab,
@@ -333,21 +332,16 @@ k_jacobian(int64_t N, const int32_t* __restrict__ cam, const int32_t* __restrict
         }
     }
     double* out = vals + 2 * base;
-    if (BULK) {
-        // 2 * base and `total` are even: source, destination and size are multiples of 16 bytes.  Every lane orders its own
-        // (generic-proxy) shared-memory stores before the asynchronous proxy's read; lane 0 then issues the copy and holds the
-        // CTA's shared memory until the unit has read it.
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncwarp();
-        if (lane == 0 && total > 0) {
-            const unsigned src = (unsigned)__cvta_generic_to_shared(ws);
-            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(out), "r"(src), "r"((unsigned)(total * 8)) : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-        }
-    } else {
-        __syncwarp();
-        for (int64_t t = lane; t < total; t += 32) out[t] = ws[t];
+    // 2 * base and `total` are even: source, destination and size are multiples of 16 bytes.  Every lane orders its own
+    // (generic-proxy) shared-memory stores before the asynchronous proxy's read; lane 0 then issues the copy and holds the
+    // CTA's shared memory until the unit has read it.
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    __syncwarp();
+    if (lane == 0 && total > 0) {
+        const unsigned src = (unsigned)__cvta_generic_to_shared(ws);
+        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(out), "r"(src), "r"((unsigned)(total * 8)) : "memory");
+        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
     }
 }
 
@@ -939,8 +933,7 @@ int pcs_jacobian_values_dev(pcs_problem* p, const double* x_dev, double* vals_de
     if (p->N == 0) return PCS_OK;
     const int grid = grid_for(p->N, 128);
     const size_t smem = (size_t)4 * 64 * p->P * sizeof(double);
-    static const bool bulk = [] { const char* e = std::getenv("PCS_JAC_BULK"); return !(e && e[0] == '0'); }();
-    auto kern = p->P == 21 ? (bulk ? k_jacobian<21, true> : k_jacobian<21, false>) : (bulk ? k_jacobian<24, true> : k_jacobian<24, false>);
+    auto kern = p->P == 21 ? k_jacobian<21> : k_jacobian<24>;
     PCS_CUDA(ensure_dynamic_smem(kern, smem));
     kern<<<grid, 128, smem, p->stream>>>(p->N, p->cam, p->pose, p->key, (const double2*)p->uv, p->camtab, p->posetab, p->dRtab,
                                          points_ptr(p), p->cam_mask, p->pose_mask, p->key_mask, p->row_prefix, p->C, vals_dev);

@@ -3,7 +3,6 @@
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdio>
-#include <cstdlib>
 #include <map>
 #include <mutex>
 #include <string>
@@ -56,18 +55,11 @@ inline cudaError_t ensure_dynamic_smem(Kernel kernel, size_t bytes)
 // before it in the stream is still running; it must call pdl_wait() before it touches anything that kernel writes (the
 // wait returns once the whole prerequisite grid has completed and flushed).  The earlier kernel allows this by calling
 // pdl_launch_dependents().  Net effect: the launch latency and the on-chip prologue of the dependent overlap the tail of
-// its predecessor.  Without the launch attribute (or with PCS_PDL=0) both instructions are no-ops and the stream
-// serialises as usual.
+// its predecessor.  Without the launch attribute both instructions are no-ops and the stream serialises as usual.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #endif
-
-inline bool pdl_enabled()
-{
-    static const bool on = [] { const char* e = std::getenv("PCS_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args)
@@ -76,7 +68,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }

@@ -278,30 +278,20 @@ struct ObsJacCam {
 
 // Table rows are fetched with 16-byte loads (rows are 16-byte aligned): camera row doubles 0..21 = q(9) R(9) t(3)
 // (+1 unused), pose row doubles 0..11 = R(9) t(3); the template row is padded to 4 doubles.
-template <bool FAKE_ROWS = false>   // FAKE_ROWS: timing experiment only (rows made up from registers, no loads)
 __device__ __forceinline__ void eval_obs_cam(const double* __restrict__ cam, const double* __restrict__ pose,
                                              const double* __restrict__ pt4, double u_obs, double v_obs, double res[2],
                                              ObsJacCam& J)
 {
     double cv[22], pv[12], Xt[4];
-    if constexpr (FAKE_ROWS) {
+    const double2* c2 = reinterpret_cast<const double2*>(cam);
+    const double2* p2 = reinterpret_cast<const double2*>(pose);
+    const double2* x2 = reinterpret_cast<const double2*>(pt4);
 #pragma unroll
-        for (int k = 0; k < 12; ++k) pv[k] = u_obs * (1e-6 * (k + 1)) + (k % 4 == 0 ? 1.0 : 0.0);
+    for (int k = 0; k < 6; ++k) { const double2 v = p2[k]; pv[2 * k] = v.x; pv[2 * k + 1] = v.y; }
 #pragma unroll
-        for (int k = 0; k < 4; ++k) Xt[k] = v_obs * (1e-6 * (k + 1));
+    for (int k = 0; k < 2; ++k) { const double2 v = x2[k]; Xt[2 * k] = v.x; Xt[2 * k + 1] = v.y; }
 #pragma unroll
-        for (int k = 0; k < 22; ++k) cv[k] = u_obs * (1e-7 * (k + 1)) + (k % 5 == 0 ? 1.0 : 0.1);
-    } else {
-        const double2* c2 = reinterpret_cast<const double2*>(cam);
-        const double2* p2 = reinterpret_cast<const double2*>(pose);
-        const double2* x2 = reinterpret_cast<const double2*>(pt4);
-#pragma unroll
-        for (int k = 0; k < 6; ++k) { const double2 v = p2[k]; pv[2 * k] = v.x; pv[2 * k + 1] = v.y; }
-#pragma unroll
-        for (int k = 0; k < 2; ++k) { const double2 v = x2[k]; Xt[2 * k] = v.x; Xt[2 * k + 1] = v.y; }
-#pragma unroll
-        for (int k = 0; k < 11; ++k) { const double2 v = c2[k]; cv[2 * k] = v.x; cv[2 * k + 1] = v.y; }
-    }
+    for (int k = 0; k < 11; ++k) { const double2 v = c2[k]; cv[2 * k] = v.x; cv[2 * k + 1] = v.y; }
     double Xw[3], Yc[3], Xc[3];
     transform(pv + POSE_R, pv + POSE_T, Xt, Xw);
     rotate(cv + CAM_R, Xw, Yc);

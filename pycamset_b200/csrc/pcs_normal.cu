@@ -27,7 +27,6 @@
 //     block inside the flushes (Jl_m folded into the adjoint, Jl_c on three rows of W_s and on U_c / g_c).
 //   HBM traffic per observation: (u,v) 16 B + camera, pose, key 12 B = 28 B read; outputs are O(segments).
 #include <algorithm>
-#include <cstdlib>
 
 #include "pcs_internal.cuh"
 #include "pcs_math.cuh"
@@ -217,29 +216,17 @@ __device__ __forceinline__ void flush_camera(int lane, int c, const double* __re
     __syncwarp();
 }
 
-// One k-step (2 observations = 4 staged rows) of the Gram update: fragment loads and the three DMMA (the knock-out
-// variants of the attribution experiment replace either by a no-op that keeps the operands alive).
-template <int KO>
+// One k-step (2 observations = 4 staged rows) of the Gram update: fragment loads and the three DMMA.
 __device__ __forceinline__ void gram_mma(NeAcc& S, double v0, double v1)
 {
-    if constexpr (KO & 1) {
-        asm volatile("" ::"d"(v0), "d"(v1));
-    } else {
-        dmma884(S.aa[0], S.aa[1], v0, v0);
-        dmma884(S.ab[0], S.ab[1], v0, v1);
-        dmma884(S.bb[0], S.bb[1], v1, v1);
-    }
+    dmma884(S.aa[0], S.aa[1], v0, v0);
+    dmma884(S.ab[0], S.ab[1], v0, v1);
+    dmma884(S.bb[0], S.bb[1], v1, v1);
 }
-template <int KO>
 __device__ __forceinline__ void gram_load(const double* __restrict__ f, double& v0, double& v1)
 {
-    if constexpr (KO & 2) {
-        v0 = __longlong_as_double((long long)(size_t)f);   // address-dependent bits: nothing is loaded
-        v1 = v0 * 0.5;
-    } else {
-        v0 = f[0];
-        v1 = f[NE_TILE_DOUBLES];
-    }
+    v0 = f[0];
+    v1 = f[NE_TILE_DOUBLES];
 }
 
 // Streamed observation loads: every observation is read exactly once per evaluation, so the loads bypass L1
@@ -275,7 +262,6 @@ __device__ __forceinline__ void load_obs(NeObs& o, int64_t i, int64_t end, const
 struct NeRows {
     double xD, yD, Au[5], Av[5], Pm[6], Wc[6], res[2];
 };
-template <bool FAKE_ROWS = false>
 __device__ __forceinline__ void eval_rows(const NeObs& o, const double* __restrict__ camtab, const double* __restrict__ posetab,
                                           const double* __restrict__ pts, NeRows& R)
 {
@@ -283,7 +269,7 @@ __device__ __forceinline__ void eval_rows(const NeObs& o, const double* __restri
     const double* ct = camtab + (int64_t)max(o.c, 0) * CAM_STRIDE;
     const double* ptab = posetab + (int64_t)max(o.m, 0) * POSE_STRIDE;
     ObsJacCam J;
-    eval_obs_cam<FAKE_ROWS>(ct, ptab, pts + 4 * (int64_t)(o.c < 0 ? 0 : o.k), o.uv.x, o.uv.y, R.res, J);
+    eval_obs_cam(ct, ptab, pts + 4 * (int64_t)(o.c < 0 ? 0 : o.k), o.uv.x, o.uv.y, R.res, J);
     R.xD = J.xD; R.yD = J.yD;
 #pragma unroll
     for (int i = 0; i < 5; ++i) { R.Au[i] = J.Au[i]; R.Av[i] = J.Av[i]; }
@@ -320,12 +306,9 @@ __device__ __forceinline__ void stage_rows(const NeRows& R, double* __restrict__
     }
 }
 
-// KO: knock-out bits of the attribution experiment (tools/kne_knockout.sh, built with -DPCS_NE_KNOCKOUT only; results are
-// wrong by construction, only the time is read): 1 = no DMMA in the Gram loop, 2 = no fragment loads, 4 = no staging
-// stores, 8 = table rows made up from registers (no row loads), 16 = no segment flush.
 // (A variant with two observations per lane and loop trip -- two independent evaluation chains -- was measured at 0.177 ms
 // against 0.135 ms: the second observation's rows spill.  Removed.)
-template <int CTAS_PER_SM, int WARPS, int KO = 0, bool PF_LATE = true>
+template <int CTAS_PER_SM, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32, CTAS_PER_SM)
 k_normal(int n_warps, const int64_t* __restrict__ warp_seg, const int32_t* __restrict__ s_cam, const int32_t* __restrict__ s_pose,
          const int32_t* __restrict__ s_key, const double2* __restrict__ s_uv, const int64_t* __restrict__ seg_start,
@@ -378,33 +361,18 @@ k_normal(int n_warps, const int64_t* __restrict__ warp_seg, const int32_t* __res
     for (int64_t base = begin; base < end; base += 32) {
         const NeObs ob = nxt;
         NeRows rows;
-        if (!PF_LATE) load_obs(nxt, base + 32 + lane, end, s_cam, s_pose, s_key, s_uv);
-        eval_rows<(KO & 8) != 0>(ob, camtab, posetab, pts, rows);
-        // PF_LATE: the next trip's stream loads are issued only now.  Issued at the top of the trip they shared a scoreboard
-        // with this trip's table-row loads, so the first use of a row waited for the whole DRAM latency of the prefetch
-        // (17 % of the warp samples sat on two such instructions); the Gram phase below is long enough to cover them:
-        // 131.1 -> 127.0 us at config 4 (a two-deep variant spills and gains nothing, nor does pulling the next trip's pose
-        // rows into L1 from pose indices loaded one trip further ahead; PCS_NE_PF_LATE=0 restores the early issue).
-        if (PF_LATE) load_obs(nxt, base + 32 + lane, end, s_cam, s_pose, s_key, s_uv);
-        // the next trip's pose rows (new for every segment) are pulled into L1 while this trip's Gram phase runs
-        if (!PF_LATE && nxt.m >= 0) {
-            const double* nx = posetab + (int64_t)nxt.m * POSE_STRIDE;
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(nx));
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(nx + 16));
-        }
+        eval_rows(ob, camtab, posetab, pts, rows);
+        // the next trip's stream loads are issued only now.  Issued at the top of the trip they shared a scoreboard with
+        // this trip's table-row loads, so the first use of a row waited for the whole DRAM latency of the prefetch (17 % of
+        // the warp samples sat on two such instructions); the Gram phase below is long enough to cover them: 131.1 -> 127.0
+        // us at config 4 (a two-deep variant spills and gains nothing, nor does pulling the next trip's pose rows into L1
+        // from pose indices loaded one trip further ahead).
+        load_obs(nxt, base + 32 + lane, end, s_cam, s_pose, s_key, s_uv);
         const int cnt = (int)min((int64_t)32, end - base);
         const int c = ob.c, m = ob.m;
         // every lane stages its rows, also the lanes past the end of the range (they evaluated row 0 of every table: finite
         // values, masked out of the Gram steps below): without a predicate the stores are free to move up into the evaluation
-        if constexpr (KO & 4) {
-            asm volatile("" ::"d"(rows.xD), "d"(rows.yD), "d"(rows.res[0]), "d"(rows.res[1]));
-#pragma unroll
-            for (int q = 0; q < 5; ++q) asm volatile("" ::"d"(rows.Au[q]), "d"(rows.Av[q]));
-#pragma unroll
-            for (int q = 0; q < 6; ++q) asm volatile("" ::"d"(rows.Pm[q]), "d"(rows.Wc[q]));
-        } else {
-            stage_rows(rows, st_u, st_v, st_rot);
-        }
+        stage_rows(rows, st_u, st_v, st_rot);
         // piece heads: lanes whose (camera, pose) differs from the previous observation's
         int pc = __shfl_up_sync(0xffffffffu, c, 1), pm = __shfl_up_sync(0xffffffffu, m, 1);
         if (lane == 0) { pc = last_c; pm = last_m; }
@@ -418,10 +386,7 @@ k_normal(int n_warps, const int64_t* __restrict__ warp_seg, const int32_t* __res
             pieces &= pieces - 1;
             const int b = pieces ? __ffs(pieces) - 1 : cnt;
             if ((heads >> a) & 1u) {
-                if (cur_c >= 0) {
-                    if constexpr (KO & 16) { asm volatile("" ::"d"(S.aa[0]), "d"(S.aa[1]), "d"(S.ab[0]), "d"(S.ab[1]), "d"(S.bb[0]), "d"(S.bb[1])); acc_zero(S); }
-                    else flush_segment(S, lane, cur_seg, cur_c, cur_m, camtab, posetab, scratch, scratch + 64, V, gp, W);
-                }
+                if (cur_c >= 0) flush_segment(S, lane, cur_seg, cur_c, cur_m, camtab, posetab, scratch, scratch + 64, V, gp, W);
                 const int nc = __shfl_sync(0xffffffffu, c, a);
                 if (nc != cur_c && cur_c >= 0) flush_camera(lane, cur_c, camtab, scratch + 64, U, gc, cost);
                 ++cur_seg; cur_c = nc; cur_m = __shfl_sync(0xffffffffu, m, a);
@@ -433,12 +398,12 @@ k_normal(int n_warps, const int64_t* __restrict__ warp_seg, const int32_t* __res
 #pragma unroll
                 for (int k4 = 0; k4 < 16; k4 += 4) {
                     double v0[4], v1[4];
-                    gram_load<KO>(fb0 + 32 * k4, v0[0], v1[0]);
-                    gram_load<KO>(fb1 + 32 * (k4 + 1), v0[1], v1[1]);
-                    gram_load<KO>(fb2 + 32 * (k4 + 2), v0[2], v1[2]);
-                    gram_load<KO>(fb3 + 32 * (k4 + 3), v0[3], v1[3]);
+                    gram_load(fb0 + 32 * k4, v0[0], v1[0]);
+                    gram_load(fb1 + 32 * (k4 + 1), v0[1], v1[1]);
+                    gram_load(fb2 + 32 * (k4 + 2), v0[2], v1[2]);
+                    gram_load(fb3 + 32 * (k4 + 3), v0[3], v1[3]);
 #pragma unroll
-                    for (int u = 0; u < 4; ++u) gram_mma<KO>(S, v0[u], v1[u]);
+                    for (int u = 0; u < 4; ++u) gram_mma(S, v0[u], v1[u]);
                 }
             } else {
                 // general piece: steps outside [a, b) are skipped (warp-uniform), steps shared with a neighbouring piece or
@@ -448,14 +413,14 @@ k_normal(int n_warps, const int64_t* __restrict__ warp_seg, const int32_t* __res
                     if (2 * ks + 2 <= a || 2 * ks >= b) continue;
                     const double* f = ((ks & 3) == 0 ? fb0 : (ks & 3) == 1 ? fb1 : (ks & 3) == 2 ? fb2 : fb3) + 32 * ks;
                     double v0, v1;
-                    gram_load<KO>(f, v0, v1);
+                    gram_load(f, v0, v1);
                     if (2 * ks < a || 2 * ks + 2 > b) {
                         const int o = 2 * ks + jb;
                         const bool ok = o >= a && o < b;
                         v0 = ok ? v0 : 0.0;
                         v1 = ok ? v1 : 0.0;
                     }
-                    gram_mma<KO>(S, v0, v1);
+                    gram_mma(S, v0, v1);
                 }
             }
         }
@@ -773,13 +738,11 @@ int launch_normal_blocks(pcs_problem* p, bool targets_cleared, int part, int n_p
     if (p->N == 0) return PCS_OK;
     // FP64 (default): 5 CTAs x 4 warps per SM, 96 registers.  Mixed (pcs_set_normal_precision): BF16-split Gram on HMMA.
     const bool mixed = p->normal_precision == PCS_PRECISION_MIXED;
-    // mixed kernel: 4 CTAs per SM (128 registers, no spills) or 5 (96 registers, 80 B of spills); PCS_NEM_CTAS for A/B runs
-    static const int nem_ctas = [] { const char* e = std::getenv("PCS_NEM_CTAS"); return e && e[0] == '5' ? 5 : 4; }();
-    const int ctas = mixed ? nem_ctas : 5, warps = 4;
+    // mixed kernel: 4 CTAs per SM (128 registers, no spills; at 5 CTAs it has 96 registers and 80 B of spills)
+    const int ctas = mixed ? 4 : 5, warps = 4;
     const size_t smem = (size_t)warps * (mixed ? NEM_WARP_DOUBLES : NE_WARP_DOUBLES) * sizeof(double);
-    auto kern_mixed = nem_ctas == 5 ? k_normal_mixed<5, 4> : k_normal_mixed<4, 4>;
-    if (mixed) PCS_CUDA(ensure_dynamic_smem(kern_mixed, smem));
-    else { PCS_CUDA(ensure_dynamic_smem(k_normal<5, 4>, smem)); PCS_CUDA(ensure_dynamic_smem(k_normal<5, 4, 0, false>, smem)); }
+    if (mixed) PCS_CUDA(ensure_dynamic_smem(k_normal_mixed<4, 4>, smem));
+    else PCS_CUDA(ensure_dynamic_smem(k_normal<5, 4>, smem));
     // persistent-style grid: `ctas` CTAs of `warps` warps per SM; at least ~64 observations per warp
     const int64_t n_part_obs = p->N / n_parts + 1;
     int64_t n_warps = std::min<int64_t>((n_part_obs + 63) / 64, (int64_t)p->sm_count * ctas * warps);
@@ -789,28 +752,8 @@ int launch_normal_blocks(pcs_problem* p, bool targets_cleared, int part, int n_p
     const int tslot = (int)(p->timing_count % (int64_t)std::max<size_t>(p->ev_a.size(), 1));
     if (p->timing) PCS_CUDA(cudaEventRecord(p->ev_a[tslot], p->stream));
     const int64_t* ranges = p->warp_seg[n_parts > 1 ? 1 : 0] + (int64_t)part * (n_warps + 1);
-    static const bool pf_early = [] { const char* e = std::getenv("PCS_NE_PF_LATE"); return e && e[0] == '0'; }();   // A/B switch
-    auto kern_fp64 = pf_early ? k_normal<5, 4, 0, false> : k_normal<5, 4>;
-#ifdef PCS_NE_KNOCKOUT
-    {
-        static const int ko = [] { const char* e = std::getenv("PCS_NE_KO"); return e ? std::atoi(e) : 0; }();
-        switch (ko) {
-            case 1: kern_fp64 = k_normal<5, 4, 1>; break;
-            case 2: kern_fp64 = k_normal<5, 4, 2>; break;
-            case 3: kern_fp64 = k_normal<5, 4, 3>; break;
-            case 4: kern_fp64 = k_normal<5, 4, 4>; break;
-            case 7: kern_fp64 = k_normal<5, 4, 7>; break;
-            case 8: kern_fp64 = k_normal<5, 4, 8>; break;
-            case 16: kern_fp64 = k_normal<5, 4, 16>; break;
-            case 23: kern_fp64 = k_normal<5, 4, 23>; break;
-            case 31: kern_fp64 = k_normal<5, 4, 31>; break;
-            default: break;
-        }
-        if (ko) PCS_CUDA(ensure_dynamic_smem(kern_fp64, smem));
-    }
-#endif
     // programmatic dependent launch: the grid becomes resident while k_prepare_tables drains (pdl_wait inside the kernel)
-    PCS_CUDA(launch_pdl(mixed ? kern_mixed : kern_fp64, dim3(grid), dim3(warps * 32), smem, p->stream, (int)n_warps, ranges,
+    PCS_CUDA(launch_pdl(mixed ? k_normal_mixed<4, 4> : k_normal<5, 4>, dim3(grid), dim3(warps * 32), smem, p->stream, (int)n_warps, ranges,
                         (const int32_t*)p->s_cam, (const int32_t*)p->s_pose, (const int32_t*)p->s_key, (const double2*)p->s_uv,
                         (const int64_t*)p->seg_start, (const double*)p->camtab, (const double*)p->posetab, (const double*)p->tmpl4,
                         p->U, p->gc, p->cost, p->V, p->gp, p->W));

@@ -2,23 +2,18 @@
 //
 // The per-evaluation exchange of the pose-sharded problem (SURVEY.md 8e) is C * 240 + 1 doubles (61 KB at C = 32):
 // a latency problem, not a bandwidth one.  Every rank owns a "symmetric" buffer that all peers have mapped (the
-// Python host allocates it with torch's symmetric-memory allocator and passes the peer pointers in): flags, then two
-// slot sets of `world` blocks each, used alternately so that a rank that races ahead never overwrites a block still
-// being read.  Three kernels implement the exchange:
-//   * k_p2p_allreduce_sentinel (default) -- "the data is the signal": empty slots hold a sentinel NaN, a rank's block is
-//     pushed into its slot at every peer with plain posted stores, and the summing threads poll their own buffer's slots
-//     until the values they need have arrived; no system fence, no flag (7.6 us per exchange at N = 2);
-//   * k_p2p_allreduce / k_p2p_allreduce_multi (PCS_P2P_SENTINEL=0) -- the fence + flag protocol of round 1, single CTA or
-//     one CTA per peer: push, system fence, raise a flag at every peer, wait for every peer's flag, sum (10.4 us).
-// All of them sum the received blocks from LOCAL memory in rank order: the result is bitwise identical on every rank.
-#include <cstdlib>
-
+// Python host allocates it with torch's symmetric-memory allocator and passes the peer pointers in): a 256-byte header,
+// then two slot sets of `world` blocks each, used alternately so that a rank that races ahead never overwrites a block
+// still being read.  The exchange (k_p2p_allreduce_sentinel) pushes a rank's block into its slot at every peer with
+// plain posted stores and polls its own buffer until the sentinel NaN in the slots it needs is replaced: no system
+// fence, no flag (7.6 us per exchange at N = 2).  The received blocks are summed from LOCAL memory in rank order: the
+// result is bitwise identical on every rank.
 #include "pcs_internal.cuh"
 
 namespace pcs {
 
 constexpr int P2P_MAX_WORLD = 16;
-constexpr int64_t P2P_FLAG_DOUBLES = 32;   // 16 x uint64 flags, padded to 256 bytes
+constexpr int64_t P2P_HEADER_DOUBLES = 32; // 256 bytes; word P2P_MAX_WORLD is the `done` counter of k_p2p_allreduce_sentinel
 constexpr int P2P_ILP = 8;                 // push: entries per thread and pass with their loads in flight together
 constexpr int P2P_SUM_ILP = 4;             // sum: entries per thread and pass (x world loads each)
 
@@ -31,156 +26,11 @@ struct P2PState {
     int rank = 0, world = 1;
     int64_t n = 0;          // doubles exchanged
     uint64_t epoch = 0;
-    bool sentinel = false;  // slots were handed over filled with the sentinel (pcs_p2p_allreduce_setup flags)
-    int* err = nullptr;     // device flag: a poll of the sentinel form timed out
+    int* err = nullptr;     // device flag: a poll timed out
 };
 
-__device__ __forceinline__ void st_release_sys(uint64_t* p, uint64_t v)
-{
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint64_t ld_acquire_sys(const uint64_t* p)
-{
-    uint64_t v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ double ld_relaxed_sys(const double* p)
-{
-    double v;
-    asm volatile("ld.relaxed.sys.global.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory");
-    return v;
-}
-
-// Push protocol: every rank WRITES its block into slot [rank] of every peer's buffer (posted NVLink stores, no read
-// round trip), fences, raises its flag at every peer, waits for all flags in its own buffer and sums the `world`
-// slots it received from local memory.  Buffer layout per rank: flags | slot 0: [world][n] | slot 1: [world][n].
-template <int WORLD>
-__global__ void __launch_bounds__(1024)
-k_p2p_allreduce(double* __restrict__ local, int64_t n, int rank, int world_rt, P2PPeers peers, uint64_t epoch)
-{
-    const int world = WORLD > 0 ? WORLD : world_rt;
-    const int tid = threadIdx.x;
-    const int64_t data = P2P_FLAG_DOUBLES + (int64_t)(epoch & 1) * world * n;
-    pdl_wait();   // launched behind the normal-equation kernel with programmatic serialisation: its sums are complete from here on
-    // P2P_ILP entries per thread and pass: all loads of a pass are in flight together (the exchange is a chain of memory
-    // round trips; one entry per trip made it 8 dependent L2 / NVLink latencies long)
-    for (int64_t i0 = 0; i0 < n; i0 += (int64_t)P2P_ILP * blockDim.x) {
-        double v[P2P_ILP];
-#pragma unroll
-        for (int u = 0; u < P2P_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            v[u] = i < n ? local[i] : 0.0;
-        }
-#pragma unroll
-        for (int u = 0; u < P2P_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            if (i < n) {
-#pragma unroll
-                for (int r = 0; r < (WORLD > 0 ? WORLD : P2P_MAX_WORLD); ++r)
-                    if (r < world) peers.buf[r][data + (int64_t)rank * n + i] = v[u];
-            }
-        }
-    }
-    __threadfence_system();
-    __syncthreads();
-    double* mine = peers.buf[rank];
-    if (tid < world) {
-        st_release_sys(reinterpret_cast<uint64_t*>(peers.buf[tid]) + rank, epoch);       // my flag in peer tid's buffer
-        const uint64_t* theirs = reinterpret_cast<const uint64_t*>(mine) + tid;           // peer tid's flag in mine
-        while (ld_acquire_sys(theirs) < epoch) { }
-    }
-    __syncthreads();
-    for (int64_t i0 = 0; i0 < n; i0 += (int64_t)P2P_SUM_ILP * blockDim.x) {
-        double s[P2P_SUM_ILP];
-#pragma unroll
-        for (int u = 0; u < P2P_SUM_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            s[u] = 0.0;
-            if (i < n) {
-#pragma unroll
-                for (int r = 0; r < (WORLD > 0 ? WORLD : P2P_MAX_WORLD); ++r)
-                    if (r < world) s[u] += ld_relaxed_sys(mine + data + (int64_t)r * n + i);   // rank order: identical bits everywhere
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < P2P_SUM_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            if (i < n) local[i] = s[u];
-        }
-    }
-}
-
-// Multi-CTA form of the same protocol for larger worlds, where one SM pushing world * n doubles over NVLink is the
-// long pole: CTA b pushes the block to peer b (16-byte stores where the alignment allows) and raises this rank's flag
-// there; the CTAs of a rank tell each other through a counter in the rank's own buffer that they are done reading
-// `local`; every CTA then waits for all flags and sums its 1/world share of the entries.
-template <int WORLD>
-__global__ void __launch_bounds__(512)
-k_p2p_allreduce_multi(double* __restrict__ local, int64_t n, int rank, int world_rt, P2PPeers peers, uint64_t epoch)
-{
-    const int world = WORLD > 0 ? WORLD : world_rt;
-    const int tid = threadIdx.x, b = blockIdx.x;   // gridDim.x == world
-    const int64_t data = P2P_FLAG_DOUBLES + (int64_t)(epoch & 1) * world * n;
-    pdl_wait();
-    {
-        double* dst = peers.buf[b] + data + (int64_t)rank * n;
-        const bool vec = ((reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(local)) & 15) == 0;
-        const int64_t n2 = vec ? n / 2 : 0;
-        for (int64_t i0 = 0; i0 < n2; i0 += (int64_t)P2P_ILP * blockDim.x) {   // loads of a pass in flight together
-            double2 v[P2P_ILP];
-#pragma unroll
-            for (int u = 0; u < P2P_ILP; ++u) {
-                const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-                if (i < n2) v[u] = reinterpret_cast<const double2*>(local)[i];
-            }
-#pragma unroll
-            for (int u = 0; u < P2P_ILP; ++u) {
-                const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-                if (i < n2) reinterpret_cast<double2*>(dst)[i] = v[u];
-            }
-        }
-        for (int64_t i = 2 * n2 + tid; i < n; i += blockDim.x) dst[i] = local[i];
-    }
-    __threadfence_system();
-    __syncthreads();
-    double* mine = peers.buf[rank];
-    if (tid == 0) {
-        st_release_sys(reinterpret_cast<uint64_t*>(peers.buf[b]) + rank, epoch);   // my flag in peer b's buffer
-        atomicAdd(reinterpret_cast<unsigned long long*>(mine) + P2P_MAX_WORLD, 1ull);   // this CTA is done reading `local`
-    }
-    if (tid < world) {
-        const uint64_t* theirs = reinterpret_cast<const uint64_t*>(mine) + tid;     // peer tid's flag in mine
-        while (ld_acquire_sys(theirs) < epoch) { }
-    } else if (tid == world) {
-        const uint64_t* done = reinterpret_cast<const uint64_t*>(mine) + P2P_MAX_WORLD;
-        while (ld_acquire_sys(done) < epoch * (uint64_t)world) { }
-    }
-    __syncthreads();
-    const int64_t e0 = n * b / world, e1 = n * (b + 1) / world;
-    for (int64_t i0 = e0; i0 < e1; i0 += (int64_t)P2P_SUM_ILP * blockDim.x) {
-        double s[P2P_SUM_ILP];
-#pragma unroll
-        for (int u = 0; u < P2P_SUM_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            s[u] = 0.0;
-            if (i < e1) {
-#pragma unroll
-                for (int r = 0; r < (WORLD > 0 ? WORLD : P2P_MAX_WORLD); ++r)
-                    if (r < world) s[u] += ld_relaxed_sys(mine + data + (int64_t)r * n + i);   // rank order: identical bits everywhere
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < P2P_SUM_ILP; ++u) {
-            const int64_t i = i0 + (int64_t)u * blockDim.x + tid;
-            if (i < e1) local[i] = s[u];
-        }
-    }
-}
-
-
-// "The data is the signal" form (default): the slots of a buffer hold a sentinel NaN whenever they are empty.  CTA b
-// pushes this rank's block into its slot at peer b -- no system fence, no flag -- and every CTA sums its 1 / world share of
+// "The data is the signal": the slots of a buffer hold a sentinel NaN whenever they are empty.  CTA b pushes this rank's
+// block into its slot at peer b -- no system fence, no flag -- and every CTA sums its 1 / world share of
 // the entries by polling the `world` slots of its OWN buffer until none of the values it needs is the sentinel (8-byte
 // stores are atomic, so a value is either the sentinel or complete), in rank order (identical bits on every rank), and
 // then puts the sentinel back.  A slot set is reused two exchanges later; the peer's write for that exchange causally
@@ -208,7 +58,7 @@ k_p2p_allreduce_sentinel(double* __restrict__ local, int64_t n, int rank, int wo
 {
     const int world = WORLD > 0 ? WORLD : world_rt;
     const int tid = threadIdx.x, b = blockIdx.x;   // gridDim.x == world
-    const int64_t data = P2P_FLAG_DOUBLES + (int64_t)(epoch & 1) * world * n;
+    const int64_t data = P2P_HEADER_DOUBLES + (int64_t)(epoch & 1) * world * n;
     pdl_wait();
     {
         double* dst = peers.buf[b] + data + (int64_t)rank * n;
@@ -291,7 +141,7 @@ int64_t pcs_p2p_buffer_bytes(const pcs_problem* p, int world)
 {
     if (!p || world < 1) return 0;
     const int64_t n = (int64_t)p->C * 240 + 1;
-    return (P2P_FLAG_DOUBLES + 2 * (int64_t)world * n) * (int64_t)sizeof(double);
+    return (P2P_HEADER_DOUBLES + 2 * (int64_t)world * n) * (int64_t)sizeof(double);
 }
 
 int pcs_p2p_allreduce_setup(pcs_problem* p, int rank, int world, void* const* peer_buffers, int64_t buffer_bytes)
@@ -309,19 +159,14 @@ int pcs_p2p_allreduce_setup(pcs_problem* p, int rank, int world, void* const* pe
         st->peers.buf[r] = (double*)peer_buffers[r];
     }
     st->rank = rank; st->world = world; st->n = (int64_t)p->C * 240 + 1; st->epoch = 0;
-    // the sentinel form needs the slots of THIS rank's buffer filled with the sentinel (done here; the caller's barrier
-    // after setup -- see pycamset_b200/distributed.py -- keeps any peer from pushing before that); PCS_P2P_SENTINEL=0
-    // selects the fence + flag protocol
-    const char* e = std::getenv("PCS_P2P_SENTINEL");
-    st->sentinel = !(e && e[0] == '0');
-    if (st->sentinel) {
-        if (!st->err) PCS_CUDA(cudaMalloc((void**)&st->err, sizeof(int)));
-        PCS_CUDA(cudaMemsetAsync(st->err, 0, sizeof(int), p->stream));
-        const int64_t n_slots = 2 * (int64_t)world * st->n;
-        k_p2p_fill_sentinel<<<(int)((n_slots + 255) / 256), 256, 0, p->stream>>>(st->peers.buf[rank] + P2P_FLAG_DOUBLES, n_slots);
-        PCS_CUDA(cudaGetLastError());
-        PCS_CUDA(cudaStreamSynchronize(p->stream));
-    }
+    // the slots of THIS rank's buffer are filled with the sentinel here; the caller's barrier after setup -- see
+    // pycamset_b200/distributed.py -- keeps any peer from pushing before that
+    if (!st->err) PCS_CUDA(cudaMalloc((void**)&st->err, sizeof(int)));
+    PCS_CUDA(cudaMemsetAsync(st->err, 0, sizeof(int), p->stream));
+    const int64_t n_slots = 2 * (int64_t)world * st->n;
+    k_p2p_fill_sentinel<<<(int)((n_slots + 255) / 256), 256, 0, p->stream>>>(st->peers.buf[rank] + P2P_HEADER_DOUBLES, n_slots);
+    PCS_CUDA(cudaGetLastError());
+    PCS_CUDA(cudaStreamSynchronize(p->stream));
     return PCS_OK;
 }
 
@@ -331,22 +176,9 @@ int pcs_p2p_allreduce_camera_blocks(pcs_problem* p)
     PCS_CUDA(cudaSetDevice(p->device));
     P2PState* st = (P2PState*)p->p2p;
     ++st->epoch;
-    auto kern = st->world == 2 ? k_p2p_allreduce<2> : st->world == 4 ? k_p2p_allreduce<4> : st->world == 8 ? k_p2p_allreduce<8>
-                                                                                                          : k_p2p_allreduce<0>;
-    // worlds of 8 and more use the multi-CTA form (PCS_P2P_MULTI=0/1 forces either one for A/B runs)
-    static const int force = [] { const char* e = std::getenv("PCS_P2P_MULTI"); return e ? (e[0] == '1' ? 1 : 0) : -1; }();
-    const bool multi = force >= 0 ? force == 1 : st->world >= 8;
-    if (st->sentinel) {
-        auto sk = st->world == 2 ? k_p2p_allreduce_sentinel<2> : st->world == 4 ? k_p2p_allreduce_sentinel<4>
-                  : st->world == 8 ? k_p2p_allreduce_sentinel<8> : k_p2p_allreduce_sentinel<0>;
-        PCS_CUDA(launch_pdl(sk, dim3(st->world), dim3(512), 0, p->stream, p->U, st->n, st->rank, st->world, st->peers, st->epoch, st->err));
-    } else if (multi) {
-        auto mk = st->world == 2 ? k_p2p_allreduce_multi<2> : st->world == 4 ? k_p2p_allreduce_multi<4>
-                  : st->world == 8 ? k_p2p_allreduce_multi<8> : k_p2p_allreduce_multi<0>;
-        PCS_CUDA(launch_pdl(mk, dim3(st->world), dim3(512), 0, p->stream, p->U, st->n, st->rank, st->world, st->peers, st->epoch));
-    } else {
-        PCS_CUDA(launch_pdl(kern, dim3(1), dim3(1024), 0, p->stream, p->U, st->n, st->rank, st->world, st->peers, st->epoch));
-    }
+    auto kern = st->world == 2 ? k_p2p_allreduce_sentinel<2> : st->world == 4 ? k_p2p_allreduce_sentinel<4>
+                : st->world == 8 ? k_p2p_allreduce_sentinel<8> : k_p2p_allreduce_sentinel<0>;
+    PCS_CUDA(launch_pdl(kern, dim3(st->world), dim3(512), 0, p->stream, p->U, st->n, st->rank, st->world, st->peers, st->epoch, st->err));
     PCS_CUDA(cudaGetLastError());
     ++p->n_launches;
     return PCS_OK;

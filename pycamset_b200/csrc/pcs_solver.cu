@@ -20,7 +20,6 @@
 //   The pose elimination skips the structurally zero blocks of Z (static unit list, pcs_schur.cu).
 // Marquardt scaling (lambda * diag(J^T J)) plays the role of x_scale='jac'; Nielsen's gain-ratio update
 // drives lambda.  Fixed parameters are rows / columns replaced by the identity.
-#include <cublas_v2.h>
 #include <cusolverDn.h>
 
 #include <algorithm>
@@ -35,7 +34,6 @@
 namespace pcs {
 
 struct LmWorkspace {
-    cublasHandle_t blas = nullptr;
     cusolverDnHandle_t solver = nullptr;
     int64_t nc = 0;          // order of the reduced system: 15 C (+ 3 K), rounded up to a multiple of 32 (identity rows) so that every
                              // tile of the Cholesky kernel is full and moves with 16-byte copies, whatever C and K are
@@ -79,14 +77,6 @@ struct LmWorkspace {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // device time of a solve (owned by the workspace: no leak on error returns)
 };
 
-#define PCS_BLAS(call)                                                                       \
-    do {                                                                                     \
-        cublasStatus_t s__ = (call);                                                         \
-        if (s__ != CUBLAS_STATUS_SUCCESS) {                                                  \
-            set_error(std::string(#call) + " -> cuBLAS status " + std::to_string((int)s__)); \
-            return PCS_ERR_CUDA;                                                             \
-        }                                                                                    \
-    } while (0)
 #define PCS_SOLVER(call)                                                                       \
     do {                                                                                       \
         cusolverStatus_t s__ = (call);                                                         \
@@ -734,7 +724,6 @@ void lm_free(pcs_problem* p)
     if (!w) return;
     // a solve that returned early on an error may have left the problem on the second output set
     if (w->ne_alt && w->ne_orig && p->ne == w->ne_alt) swap_normal_buffers(p, w);
-    if (w->blas) cublasDestroy(w->blas);
     if (w->solver) cusolverDnDestroy(w->solver);
     schur_plan_free(&w->plan);
     if (w->seg_of) cudaFree(w->seg_of);
@@ -767,21 +756,14 @@ static int lm_prepare(pcs_problem* p)
     return rc;
 }
 
-// The library handles are created only where a library path is actually taken (the dense self-calibration fallback, a
-// reduced system too large for the persistent Cholesky kernel, or the PCS_LM_CHOL / PCS_LM_SYRK A/B switches): creating
-// them costs tens to hundreds of milliseconds per problem, more than a whole solve of a small calibration.
+// The cuSOLVER handle is created only where the library path is actually taken (the dense self-calibration fallback, a
+// reduced system too large for the persistent Cholesky kernel, or the PCS_LM_CHOL A/B switch): creating it costs tens to
+// hundreds of milliseconds per problem, more than a whole solve of a small calibration.
 static int ensure_solver(pcs_problem* p, LmWorkspace* w)
 {
     if (w->solver) return PCS_OK;
     PCS_SOLVER(cusolverDnCreate(&w->solver));
     PCS_SOLVER(cusolverDnSetStream(w->solver, p->stream));
-    return PCS_OK;
-}
-static int ensure_blas(pcs_problem* p, LmWorkspace* w)
-{
-    if (w->blas) return PCS_OK;
-    PCS_BLAS(cublasCreate(&w->blas));
-    PCS_BLAS(cublasSetStream(w->blas, p->stream));
     return PCS_OK;
 }
 
@@ -920,11 +902,7 @@ static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
         k_lm_point_Z<<<grid_for((int64_t)p->M * p->K * 3, 256), 256, 0, st>>>(p->M, p->K, nc, 15 * (int64_t)p->C, p->Ymk, w->L, w->y,
                                                                              p->pose_mask, p->key_mask, w->plan.pose_slot, w->Z, rhs);
     PCS_CUDA(cudaGetLastError());
-    const double minus1 = -1.0, one = 1.0;
-    static const bool lib_syrk = [] { const char* e = std::getenv("PCS_LM_SYRK"); return e && e[0] == 'c'; }();   // A/B runs
-    if (lib_syrk) PCS_TRY(ensure_blas(p, w));
-    if (lib_syrk) PCS_BLAS(cublasDsyrk(w->blas, CUBLAS_FILL_MODE_LOWER, CUBLAS_OP_N, (int)nc, (int)np, &minus1, w->Z, (int)nc, &one, Smat, (int)nc));
-    else PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, &w->plan));
+    PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, &w->plan));
     if (p->allreduce) {
         int rc = p->allreduce(p->allreduce_user, w->red, w->red_doubles, 0, (void*)st);
         if (rc != 0) { set_error("all-reduce callback failed"); return PCS_ERR_CUDA; }

@@ -44,8 +44,7 @@ def main():
     timed_out = prob.p2p_timed_out()
     if rank == 0:
         with open(out, "w") as f:
-            json.dump({"rel_err": worst, "timed_out": bool(timed_out), "world": world,
-                       "protocol": os.environ.get("PCS_P2P_SENTINEL", "1")}, f)
+            json.dump({"rel_err": worst, "timed_out": bool(timed_out), "world": world}, f)
     prob.close()
     dist.destroy_process_group()
 

@@ -1,6 +1,6 @@
 """Kernel time of the fused normal-equation kernel on config 4 (device-resident, L2 flushed between calls), for A/B runs
-of build variants and the knock-out attribution experiment (PCS_NE_KO, see csrc/pcs_normal.cu).
-Usage: [PCS_NE_KO=k] [KNE_MIXED=1] [KNE_RIG=C,M,layout,detect_prob] python tools/kne_ab.py"""
+of build variants.
+Usage: [KNE_MIXED=1] [KNE_RIG=C,M,layout,detect_prob] python tools/kne_ab.py"""
 import sys, os, json
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -32,5 +32,5 @@ with torch.cuda.stream(stream):
     torch.cuda.synchronize()
 ms = float(np.median(prob.timing_all_ms()))
 b = prob.device_buffers()
-print(json.dumps({"ko": os.environ.get("PCS_NE_KO"), "mixed": os.environ.get("KNE_MIXED"), "rig": spec, "n_obs": N, "kernel_ms": ms,
+print(json.dumps({"mixed": os.environ.get("KNE_MIXED"), "rig": spec, "n_obs": N, "kernel_ms": ms,
                   "Gobs_per_s": N / ms / 1e6, "frac_hbm_28B": 28.0 * N / ms / 1e6 / 6544.7}))
