@@ -238,6 +238,32 @@ PCS_API void pcs_lm_default_options(pcs_lm_options* o);
 PCS_API int pcs_lm_solve(pcs_problem* p, const double* x0 /*[n_free]*/, const pcs_lm_options* opts,
                          double* x_out /*[n_free]*/, pcs_lm_stats* stats);
 
+/* Parameter covariance at x (host buffers; x == NULL: the current parameters).  With H = J^T J over the free parameters,
+ * r the residual and N the number of observations, the unit-weight covariance Sigma = H^-1 is returned in parts:
+ *   cam   [15 C][15 C]  the full camera block, camera-major, 15 entries per camera (9 intrinsics, then 6 extrinsics: the
+ *                       layout of U);
+ *   pose  [M][6][6]     the marginal block of every pose;
+ *   point [K][3][3]     the marginal block of every target point (self-calibration chain only; ignored otherwise);
+ *   s2                  r.r / dof, dof = 2 N - (number of observed free parameters); NaN when dof <= 0;
+ *   dof.
+ * The covariance of the estimate is s2 * Sigma.  Any output may be NULL.  Camera x pose and camera x point
+ * cross-covariances are not returned (O(C M) numbers).
+ * An entry is exactly 0 when either of its parameters is fixed; otherwise NaN when either is unobserved (a free parameter
+ * whose diagonal of J^T J is zero).  Unobserved parameters are decoupled from all others: no other entry depends on them.
+ * Sigma comes from the factors of the LM solver's reduced system at lambda = 0 (S = A - Z Z^T = L L^T, Z = W L_b^-T):
+ *   reduced set    S^-1 = X^T X,                     X = L^-1;
+ *   eliminated set L_b^-T (I + X_b^T X_b) L_b^-1,    X_b = L^-1 Z_b
+ * (csrc/pcs_cov.cu).  The eliminated set is the poses, or on the self-calibration chain the points when 3 K > 6 M.
+ * The normal equations are always FP64, whatever pcs_set_normal_precision selects (the setting is kept).
+ * Side effects: those of pcs_normal_equations(p, x, NULL, ...): the parameters become x and the device block buffers hold
+ * the evaluation at x; a later pcs_lm_solve behaves as it would without this call.
+ * Errors: PCS_ERR_NUMERIC when the undamped reduced system or an eliminated block is not positive definite (typically: the
+ * gauge is not fixed); PCS_ERR_UNSUPPORTED with an all-reduce hook of world size > 1, and on the dense self-calibration
+ * fallback (no point tables, or PCS_LM_SELFCAL=dense).
+ * No reference counterpart: with scipy's solver the covariance comes from result.jac (optimisation_handling.py:52-117). */
+PCS_API int pcs_covariance(pcs_problem* p, const double* x /*[n_free] or NULL*/, double* cam, double* pose, double* point,
+                           double* s2, int64_t* dof);
+
 /* Dense symmetric positive definite solve S x = b with the persistent tiled Cholesky kernel that pcs_lm_solve uses for
  * the reduced camera system (the counterpart of the LSMR solve inside scipy's TRF, optimisation_handling.py:88-98).
  * Host buffers; A is column-major [n][n], only the lower triangle is read.  *info: 0 ok, 1 not positive definite.

@@ -21,7 +21,7 @@ EXPORTED_SYMBOLS = [
     "pcs_set_param_string", "pcs_set_free", "pcs_get_param_string", "pcs_residual", "pcs_residual_dev",
     "pcs_csr_structure", "pcs_jacobian_values", "pcs_jacobian_values_dev", "pcs_segments", "pcs_normal_equations",
     "pcs_normal_equations_dev", "pcs_point_blocks", "pcs_normal_dense", "pcs_device_buffers_get", "pcs_set_allreduce",
-    "pcs_lm_default_options", "pcs_lm_solve", "pcs_spd_solve", "pcs_syrk_sub", "pcs_lm_schur_fraction", "pcs_timing_enable", "pcs_timing_get", "pcs_timing_get_all", "pcs_launch_count",
+    "pcs_lm_default_options", "pcs_lm_solve", "pcs_covariance", "pcs_spd_solve", "pcs_syrk_sub", "pcs_lm_schur_fraction", "pcs_timing_enable", "pcs_timing_get", "pcs_timing_get_all", "pcs_launch_count",
     "pcs_costfn", "pcs_gauge_scale", "pcs_set_normal_precision", "pcs_p2p_buffer_bytes", "pcs_p2p_allreduce_setup", "pcs_p2p_allreduce_camera_blocks", "pcs_p2p_status", "pcs_device_sm_count",
     "pcs_version",
 ]
@@ -112,6 +112,7 @@ def load() -> ct.CDLL:
     lib.pcs_set_allreduce.argtypes = [vp, ALLREDUCE_FN, vp, ct.c_int, ct.c_int]
     lib.pcs_lm_default_options.argtypes = [ct.POINTER(LmOptions)]
     lib.pcs_lm_solve.argtypes = [vp, vp, ct.POINTER(LmOptions), vp, ct.POINTER(LmStats)]
+    lib.pcs_covariance.argtypes = [vp, vp, vp, vp, vp, ct.POINTER(ct.c_double), i64p]
     lib.pcs_spd_solve.argtypes = [ct.c_int, ct.c_int64, vp, vp, vp, ct.POINTER(ct.c_int)]
     lib.pcs_syrk_sub.argtypes = [ct.c_int, ct.c_int64, ct.c_int64, vp, vp]
     lib.pcs_lm_schur_fraction.argtypes = [vp, ct.POINTER(ct.c_double)]

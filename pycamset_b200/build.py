@@ -12,7 +12,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libpcs_b200.so"
-SOURCES = ["pcs_core.cu", "pcs_normal.cu", "pcs_solver.cu", "pcs_p2p.cu", "pcs_costfn.cu", "pcs_chol.cu", "pcs_schur.cu", "pcs_gauge.cu"]
+SOURCES = ["pcs_core.cu", "pcs_normal.cu", "pcs_solver.cu", "pcs_p2p.cu", "pcs_costfn.cu", "pcs_chol.cu", "pcs_schur.cu", "pcs_gauge.cu", "pcs_cov.cu"]
 HEADERS = ["pcs_math.cuh", "pcs_internal.cuh", "../../include/pcs_b200.h"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -184,4 +184,10 @@ int chol_prepare(int device, int64_t n, double** Ldiag, unsigned long long** bar
 int launch_chol_solve(cudaStream_t st, int grid, int64_t n, double* A, int64_t ld, double* rhs, double* Ldiag,
                       unsigned long long* bar, unsigned long long* bar_base, int* info, long long* trace = nullptr);
 void p2p_free(pcs_problem* p);
+// pcs_cov.cu: covariance from the factored reduced system (S off-diagonal tiles of L, Ldiag its diagonal tiles)
+int cov_forward_substitution(cudaStream_t st, int64_t nc, const double* S, double* Ldiag, double* Xi, double* Z, int64_t np);
+int cov_reduced_inverse(cudaStream_t st, int sm_count, int64_t nc, double* Xi, double* S);
+int cov_block_marginals(cudaStream_t st, int n_blocks, int B, int64_t nc, const double* X, const int32_t* slot, double* L);
+int cov_assemble(cudaStream_t st, const pcs_problem* p, int64_t nc, int red_B, int elim_B, const double* S, double* elim,
+                 double* out_cam, double* out_red, double* n_observed);
 }  // namespace pcs

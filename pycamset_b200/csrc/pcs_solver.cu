@@ -75,6 +75,12 @@ struct LmWorkspace {
     double* Hd = nullptr;    // damped copy [n_free^2]
     double* rhs = nullptr;   // [n_free]
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // device time of a solve (owned by the workspace: no leak on error returns)
+    // pcs_covariance: X_I = L^-1 [nc][nc], and a Cholesky-kernel state of its own when the LM path factors with cuSOLVER
+    double* cov_Xi = nullptr;
+    double* cov_Ldiag = nullptr;
+    unsigned long long* cov_bar = nullptr;
+    unsigned long long cov_bar_base = 0;
+    int cov_grid = 0;
 };
 
 #define PCS_SOLVER(call)                                                                       \
@@ -728,10 +734,12 @@ void lm_free(pcs_problem* p)
     schur_plan_free(&w->plan);
     if (w->seg_of) cudaFree(w->seg_of);
     if (w->dck) cudaFree(w->dck);
-    double* ptrs[] = {w->L, w->y, w->Z, w->red, w->delta, w->backup, w->scal, w->work, w->Hd, w->rhs, w->Ldiag, w->ne_alt};
+    double* ptrs[] = {w->L, w->y, w->Z, w->red, w->delta, w->backup, w->scal, w->work, w->Hd, w->rhs, w->Ldiag, w->ne_alt,
+                      w->cov_Xi, w->cov_Ldiag};
     for (double* q : ptrs) if (q) cudaFree(q);
     if (w->info) cudaFree(w->info);
     if (w->bar) cudaFree(w->bar);
+    if (w->cov_bar) cudaFree(w->cov_bar);
     if (w->h_read) cudaFreeHost(w->h_read);
     if (w->d_read) cudaFree(w->d_read);
     if (w->comb) cudaFree(w->comb);
@@ -843,46 +851,11 @@ static int eval_normal(pcs_problem* p)
     return PCS_OK;
 }
 
-// Self-calibration chain, points eliminated (w->pts_elim): same contract as solve_template below.
-static int solve_points_eliminated(pcs_problem* p, LmWorkspace* w, double lambda)
-{
-    cudaStream_t st = p->stream;
-    const int64_t nc = w->nc, np = w->np, n_cam = 15 * (int64_t)p->C;
-    double* Smat = w->red;
-    double* rhs = w->red + nc * nc;
-    double* gcopy = rhs + nc;
-    double* cost_r = gcopy + nc;
-    k_lm_init_reduced_cp<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, p->M, nc, w->nl, lambda, p->U, p->gc, p->V, p->gp, p->W,
-                                                                                     w->seg_of, p->cost, p->cam_mask, p->pose_mask, Smat, rhs,
-                                                                                     gcopy, cost_r, w->scal, w->info);
-    k_lm_point_factor<<<grid_for(p->K, 128), 128, 0, st>>>(p->K, lambda, p->Pk, p->gk, p->key_mask, w->L, w->y, w->scal);
-    k_lm_point_elim_Z<<<dim3(grid_for(nc, 128), (p->K + PT_CHUNK - 1) / PT_CHUNK), 128, 0, st>>>(p->C, p->M, p->K, nc, w->nl, p->Xck, p->Ymk, w->L,
-                                                                                              w->y, p->cam_mask, p->pose_mask, p->key_mask, w->Z, rhs);
-    PCS_CUDA(cudaGetLastError());
-    PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, nullptr));
-    k_lm_fix_diag<<<grid_for(nc, 256), 256, 0, st>>>(nc, Smat);
-    if (w->chol_grid > 0) {
-        PCS_TRY(launch_chol_solve(st, w->chol_grid, nc, Smat, nc, rhs, w->Ldiag, w->bar, &w->bar_base, w->info));
-    } else {
-        PCS_SOLVER(cusolverDnDpotrf(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, Smat, (int)nc, w->work, w->lwork, w->info));
-        PCS_SOLVER(cusolverDnDpotrs(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, 1, Smat, (int)nc, rhs, (int)nc, w->info));
-    }
-    p->n_launches += 7;
-    // rhs now holds [delta_c | delta_m]; the points follow from the back substitution
-    PCS_CUDA(cudaMemcpyAsync(w->dck, rhs, (size_t)n_cam * 8, cudaMemcpyDeviceToDevice, st));
-    k_lm_point_back<<<grid_for((int64_t)p->K * 32, 128), 128, 0, st>>>(p->K, nc, w->L, w->y, w->Z, rhs, w->dck + n_cam);
-    const int K3 = 3 * p->K;
-    k_lm_assemble_delta<<<grid_for(n_cam + 6 * (int64_t)p->M + K3, 128), 128, 0, st>>>(
-        p->C, p->M, K3, lambda, w->dck, rhs + n_cam, p->U, p->gc, p->V, p->gp, p->Pk, p->gk, p->cam_mask, p->pose_mask, p->key_mask, p->params,
-        w->delta, w->scal, 1, 1);
-    PCS_CUDA(cudaGetLastError());
-    return PCS_OK;
-}
-
-// One damped solve at the current linearisation, enqueued without synchronising.  Afterwards w->delta holds the step
-// (parameter-string layout), w->scal = {pred, |dx|^2, |x|^2, |g_pose|_inf, |g_cam|_inf, flag, trial cost, -},
-// w->info the factorisation status and cost_r (inside w->red) the all-reduced r.r of the linearisation point.
-static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
+// The reduced system at damping lambda, built in w->red and ready for the factorisation: S (lower triangle; fixed and
+// unobserved unknowns are identity rows), rhs = -g_red - Z y, the gradient copy and the cost; w->L / w->y hold the
+// eliminated blocks' Cholesky factors and L_b^-1 (-g_b), w->Z the coupling W L_b^-T.  Multi-rank: S | rhs | g | cost are
+// all-reduced here.  The first half of every LM step, and what pcs_covariance factors at lambda = 0.
+static int build_reduced(pcs_problem* p, LmWorkspace* w, double lambda)
 {
     cudaStream_t st = p->stream;
     const int64_t nc = w->nc, np = w->np;
@@ -890,6 +863,18 @@ static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
     double* rhs = w->red + nc * nc;
     double* gcopy = rhs + nc;
     double* cost_r = gcopy + nc;
+    if (w->pts_elim) {   // self-calibration chain, points eliminated
+        k_lm_init_reduced_cp<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, p->M, nc, w->nl, lambda, p->U, p->gc, p->V, p->gp, p->W,
+                                                                                         w->seg_of, p->cost, p->cam_mask, p->pose_mask, Smat, rhs,
+                                                                                         gcopy, cost_r, w->scal, w->info);
+        k_lm_point_factor<<<grid_for(p->K, 128), 128, 0, st>>>(p->K, lambda, p->Pk, p->gk, p->key_mask, w->L, w->y, w->scal);
+        k_lm_point_elim_Z<<<dim3(grid_for(nc, 128), (p->K + PT_CHUNK - 1) / PT_CHUNK), 128, 0, st>>>(p->C, p->M, p->K, nc, w->nl, p->Xck, p->Ymk, w->L,
+                                                                                                  w->y, p->cam_mask, p->pose_mask, p->key_mask, w->Z, rhs);
+        PCS_CUDA(cudaGetLastError());
+        PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, nullptr));
+        k_lm_fix_diag<<<grid_for(nc, 256), 256, 0, st>>>(nc, Smat);
+        return PCS_OK;
+    }
     const bool selfcal = p->chain == PCS_CHAIN_SELFCAL;
     k_lm_init_reduced<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, p->K, nc, w->nl, lambda, p->U, p->gc, p->cost, p->cam_mask,
                                                                                   p->Pk, p->gk, p->Xck, p->key_mask,
@@ -908,12 +893,56 @@ static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
         if (rc != 0) { set_error("all-reduce callback failed"); return PCS_ERR_CUDA; }
     }
     k_lm_fix_diag<<<grid_for(nc, 256), 256, 0, st>>>(nc, Smat);
+    return PCS_OK;
+}
+
+// S = L L^T and rhs <- S^-1 rhs (the Cholesky kernel leaves the off-diagonal tiles of L in S, the diagonal ones in Ldiag)
+static int factor_solve_reduced(pcs_problem* p, LmWorkspace* w)
+{
+    cudaStream_t st = p->stream;
+    const int64_t nc = w->nc;
+    double* Smat = w->red;
+    double* rhs = w->red + nc * nc;
     if (w->chol_grid > 0) {
         PCS_TRY(launch_chol_solve(st, w->chol_grid, nc, Smat, nc, rhs, w->Ldiag, w->bar, &w->bar_base, w->info));
     } else {
         PCS_SOLVER(cusolverDnDpotrf(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, Smat, (int)nc, w->work, w->lwork, w->info));
         PCS_SOLVER(cusolverDnDpotrs(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, 1, Smat, (int)nc, rhs, (int)nc, w->info));
     }
+    return PCS_OK;
+}
+
+// Self-calibration chain, points eliminated (w->pts_elim): same contract as solve_template below.
+static int solve_points_eliminated(pcs_problem* p, LmWorkspace* w, double lambda)
+{
+    cudaStream_t st = p->stream;
+    const int64_t nc = w->nc, n_cam = 15 * (int64_t)p->C;
+    double* rhs = w->red + nc * nc;
+    PCS_TRY(build_reduced(p, w, lambda));
+    PCS_TRY(factor_solve_reduced(p, w));
+    p->n_launches += 7;
+    // rhs now holds [delta_c | delta_m]; the points follow from the back substitution
+    PCS_CUDA(cudaMemcpyAsync(w->dck, rhs, (size_t)n_cam * 8, cudaMemcpyDeviceToDevice, st));
+    k_lm_point_back<<<grid_for((int64_t)p->K * 32, 128), 128, 0, st>>>(p->K, nc, w->L, w->y, w->Z, rhs, w->dck + n_cam);
+    const int K3 = 3 * p->K;
+    k_lm_assemble_delta<<<grid_for(n_cam + 6 * (int64_t)p->M + K3, 128), 128, 0, st>>>(
+        p->C, p->M, K3, lambda, w->dck, rhs + n_cam, p->U, p->gc, p->V, p->gp, p->Pk, p->gk, p->cam_mask, p->pose_mask, p->key_mask, p->params,
+        w->delta, w->scal, 1, 1);
+    PCS_CUDA(cudaGetLastError());
+    return PCS_OK;
+}
+
+// One damped solve at the current linearisation, enqueued without synchronising.  Afterwards w->delta holds the step
+// (parameter-string layout), w->scal = {pred, |dx|^2, |x|^2, |g_pose|_inf, |g_cam|_inf, flag, trial cost, -},
+// w->info the factorisation status and cost_r (inside w->red) the all-reduced r.r of the linearisation point.
+static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
+{
+    cudaStream_t st = p->stream;
+    const int64_t nc = w->nc;
+    double* rhs = w->red + nc * nc;
+    const bool selfcal = p->chain == PCS_CHAIN_SELFCAL;
+    PCS_TRY(build_reduced(p, w, lambda));
+    PCS_TRY(factor_solve_reduced(p, w));
     p->n_launches += 8;
     // rhs now holds delta_c
     double* dp = w->delta + 15 * (int64_t)p->C;  // pose part of the parameter-string delta is written in place
@@ -1134,6 +1163,105 @@ int pcs_lm_schur_fraction(pcs_problem* p, double* fraction)
     const LmWorkspace* w = (const LmWorkspace*)p->lm_ws;
     *fraction = w->plan.units ? w->plan.fraction : 1.0;
     return PCS_OK;
+}
+
+static int covariance_impl(pcs_problem* p, const double* x, double* cam, double* pose, double* point, double* s2, int64_t* dof)
+{
+    PCS_CUDA(cudaSetDevice(p->device));
+    if (p->world > 1) {
+        set_error("pcs_covariance: the covariance is single-rank (an all-reduce hook is installed)");
+        return PCS_ERR_UNSUPPORTED;
+    }
+    if (p->chain == PCS_CHAIN_SELFCAL && !p->Pk) {
+        set_error("pcs_covariance: the dense self-calibration fallback has no block path to factor");
+        return PCS_ERR_UNSUPPORTED;
+    }
+    PCS_TRY(lm_prepare(p));
+    LmWorkspace* w = (LmWorkspace*)p->lm_ws;
+    if (w->nc == 0) {   // PCS_LM_SELFCAL=dense
+        set_error("pcs_covariance: the dense self-calibration fallback has no block path to factor");
+        return PCS_ERR_UNSUPPORTED;
+    }
+    cudaStream_t st = p->stream;
+    const int64_t nc = w->nc, np = w->np, n_cam = 15 * (int64_t)p->C;
+    if (!w->cov_Xi) PCS_CUDA(cudaMalloc((void**)&w->cov_Xi, (size_t)(nc * nc) * 8));
+    // the factor is always the Cholesky kernel's (off-diagonal tiles of L in S, diagonal tiles in Ldiag), whichever
+    // factorisation the LM path uses
+    double* Ldiag = w->Ldiag;
+    unsigned long long* bar = w->bar;
+    unsigned long long* bar_base = &w->bar_base;
+    int grid = w->chol_grid;
+    if (grid == 0) {
+        if (!w->cov_Ldiag) {
+            PCS_TRY(chol_prepare(p->device, nc, &w->cov_Ldiag, &w->cov_bar, &w->cov_grid));
+            if (w->cov_grid == 0) {
+                set_error("pcs_covariance: the reduced system is too large for the Cholesky kernel on this device");
+                return PCS_ERR_UNSUPPORTED;
+            }
+        }
+        Ldiag = w->cov_Ldiag; bar = w->cov_bar; bar_base = &w->cov_bar_base; grid = w->cov_grid;
+    }
+    if (x && p->n_free > 0) {
+        PCS_TRY(ensure_pinned(p, p->n_free));
+        std::memcpy(p->h_pin, x, (size_t)p->n_free * 8);
+        PCS_CUDA(cudaMemcpyAsync(p->x, p->h_pin, (size_t)p->n_free * 8, cudaMemcpyHostToDevice, st));
+        PCS_TRY(launch_scatter_x(p, p->x));
+    }
+    // FP64 normal equations whatever precision the LM iterations use
+    const int precision = p->normal_precision;
+    p->normal_precision = PCS_PRECISION_FP64;
+    const int rc_eval = eval_normal(p);
+    p->normal_precision = precision;
+    PCS_TRY(rc_eval);
+    double* Smat = w->red;
+    PCS_TRY(build_reduced(p, w, 0.0));
+    PCS_TRY(launch_chol_solve(st, grid, nc, Smat, nc, w->red + nc * nc, Ldiag, bar, bar_base, w->info));
+    // X = L^-1 [I | Z] in place (Z's columns become X_b), then Sigma_red = X_I^T X_I into S (negated), Sigma_bb over L_b
+    PCS_TRY(cov_forward_substitution(st, nc, Smat, Ldiag, w->cov_Xi, w->Z, np));
+    PCS_TRY(cov_reduced_inverse(st, p->sm_count, nc, w->cov_Xi, Smat));
+    const int elim_B = w->pts_elim ? 3 : 6;
+    const int n_elim = w->pts_elim ? p->K : p->M;
+    PCS_TRY(cov_block_marginals(st, n_elim, elim_B, nc, w->Z, w->pts_elim ? nullptr : w->plan.pose_slot, w->L));
+    // copy-out layout in the (now free) X_I buffer: cam [15 C][15 C], then the reduced set's pose or point blocks
+    const int red_B = w->pts_elim ? 6 : (p->chain == PCS_CHAIN_SELFCAL ? 3 : 0);
+    double* out_cam = w->cov_Xi;
+    double* out_red = w->cov_Xi + n_cam * n_cam;
+    double* n_obs = w->scal + 7;   // cleared by the reduced-system build
+    PCS_TRY(cov_assemble(st, p, nc, red_B, elim_B, Smat, w->L, out_cam, out_red, n_obs));
+    // the LM path clears Z once and relies on its static zero pattern
+    PCS_CUDA(cudaMemsetAsync(w->Z, 0, (size_t)(nc * np) * 8, st));
+    double* h = w->h_read;
+    PCS_CUDA(cudaMemcpyAsync(h, w->scal, 8 * 8, cudaMemcpyDeviceToHost, st));
+    PCS_CUDA(cudaMemcpyAsync(h + 8, w->info, sizeof(int), cudaMemcpyDeviceToHost, st));
+    PCS_CUDA(cudaMemcpyAsync(h + 9, p->cost, 8, cudaMemcpyDeviceToHost, st));
+    PCS_CUDA(cudaStreamSynchronize(st));
+    int info = 0;
+    std::memcpy(&info, h + 8, sizeof(int));
+    if (info == -2) {
+        set_error("pcs_covariance: the Cholesky kernel's grid barrier timed out");
+        return PCS_ERR_CUDA;
+    }
+    if (info != 0 || h[5] != 0.0) {
+        set_error("pcs_covariance: the undamped normal equations are not positive definite (is the gauge fixed?)");
+        return PCS_ERR_NUMERIC;
+    }
+    const int64_t d = 2 * p->N - (int64_t)h[7];
+    if (dof) *dof = d;
+    if (s2) *s2 = d > 0 ? h[9] / (double)d : std::nan("");
+    if (cam) PCS_CUDA(cudaMemcpyAsync(cam, out_cam, (size_t)(n_cam * n_cam) * 8, cudaMemcpyDeviceToHost, st));
+    double* pose_src = w->pts_elim ? out_red : (double*)w->L;
+    double* point_src = w->pts_elim ? (double*)w->L : out_red;
+    if (pose && p->M) PCS_CUDA(cudaMemcpyAsync(pose, pose_src, (size_t)p->M * 36 * 8, cudaMemcpyDeviceToHost, st));
+    if (point && p->chain == PCS_CHAIN_SELFCAL && p->K)
+        PCS_CUDA(cudaMemcpyAsync(point, point_src, (size_t)p->K * 9 * 8, cudaMemcpyDeviceToHost, st));
+    PCS_CUDA(cudaStreamSynchronize(st));
+    return PCS_OK;
+}
+
+int pcs_covariance(pcs_problem* p, const double* x, double* cam, double* pose, double* point, double* s2, int64_t* dof)
+{
+    PCS_REQUIRE(p, "NULL argument");
+    return covariance_impl(p, x, cam, pose, point, s2, dof);
 }
 
 int pcs_lm_solve(pcs_problem* p, const double* x0, const pcs_lm_options* opts_in, double* x_out, pcs_lm_stats* stats)

@@ -158,6 +158,25 @@ class GpuBundleHandler:
         x = self._load(x0)
         return self.problem.lm_solve(x, max_iter=max_nfev, ftol=ftol, xtol=xtol, gtol=gtol, verbose=verbose)
 
+    def covariance(self, x):
+        """Covariance of the least-squares estimate at x (the reference's free vector): the unit-weight blocks of
+        BundleProblem.covariance scaled by s2 = r.r / dof -- cam (15 C, 15 C), pose (M, 6, 6), point (K, 3, 3;
+        self-calibration chain) -- with s2, dof and `param_std`, the standard deviation of every entry of x in x order
+        (NaN for a parameter no observation depends on)."""
+        cov = self.problem.covariance(self._load(x))
+        s2 = cov["s2"]
+        out = {k: s2 * cov[k] for k in ("cam", "pose", "point") if k in cov}
+        C, M = self.n_cams, self.n_poses
+        var = np.zeros(self.problem.n_params)
+        d = np.diagonal(cov["cam"]).reshape(C, 15)
+        var[:9 * C] = d[:, :9].ravel()
+        var[9 * C:15 * C] = d[:, 9:].ravel()
+        var[15 * C:15 * C + 6 * M] = np.diagonal(cov["pose"], axis1=1, axis2=2).ravel()
+        if "point" in cov:
+            var[15 * C + 6 * M:] = np.diagonal(cov["point"], axis1=1, axis2=2).ravel()
+        out.update(s2=s2, dof=cov["dof"], param_std=np.sqrt(s2 * var[self.unfixed]))
+        return out
+
     def get_camset(self, x):
         """The reference handler's own get_camset(x) (camera objects are the reference's).  For the self-calibration
         handler its post-solve gauge transform (standard_bundle_handler.py:339-410) is routed through
@@ -190,7 +209,7 @@ JAC_AUTO_LIMIT_BYTES = 2 << 30   # jac="auto": the explicit CSR Jacobian is form
 
 
 def run_bundle_adjustment(param_handler, threads: int = 1, device: int = 0, solver: str = "lm", ftol=1e-8, xtol=1e-8,
-                          gtol=1e-8, jac="auto"):
+                          gtol=1e-8, jac="auto", covariance=False):
     """Drop-in for optimisation_handling.run_bundle_adjustment (:52-117): returns (result, camset).
 
     solver="lm"    Levenberg-Marquardt on the device (block normal equations + Schur complement).
@@ -204,7 +223,10 @@ def run_bundle_adjustment(param_handler, threads: int = 1, device: int = 0, solv
     False = never, "auto" = only below JAC_AUTO_LIMIT_BYTES of CSR values.  When it is skipped `result.jac` is None (the
     reference's save_camset then omits it, as it does for any result without a usable Jacobian) and
     `result.normal_blocks` holds the block diagonal of J^T J at the solution instead -- U [C][15][15], V [M][6][6], gc,
-    gp, cost: O(C + M) numbers."""
+    gp, cost: O(C + M) numbers.
+
+    covariance=True: `result["covariance"]` holds GpuBundleHandler.covariance(result.x) -- the scaled covariance blocks,
+    s2, dof and the standard deviation of every free parameter -- for either solver."""
     gpu = param_handler if isinstance(param_handler, GpuBundleHandler) else GpuBundleHandler(param_handler, device=device)
     handler = gpu.handler
     loss_fn, jac_fn = gpu.make_loss_fun(threads), gpu.make_loss_jac(threads)
@@ -234,6 +256,8 @@ def run_bundle_adjustment(param_handler, threads: int = 1, device: int = 0, solv
             result["normal_blocks"] = {k: ne[k] for k in ("U", "gc", "V", "gp", "cost")}
     else:
         raise ValueError("solver must be 'lm' or 'scipy'")
+    if covariance:
+        result["covariance"] = gpu.covariance(result.x)
     end = time.time()
     final_euclid = float(np.mean(np.linalg.norm(np.reshape(result.fun, (-1, 2)), axis=1)))
     logging.info(f"Final Euclidean error: {final_euclid:.2f} px")

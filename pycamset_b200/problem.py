@@ -298,6 +298,21 @@ class BundleProblem:
         self._cb = L.ALLREDUCE_FN(_cb)
         L.check(self._lib.pcs_set_allreduce(self._h, self._cb, None, int(rank), int(world_size)))
 
+    def covariance(self, x=None):
+        """Unit-weight covariance H^-1 (H = J^T J over the free parameters) at x (None: the current parameters), in the
+        parts pcs_covariance returns: cam (15 C, 15 C), pose (M, 6, 6), point (K, 3, 3; self-calibration chain), the
+        residual variance s2 = r.r / dof and dof.  Entries of fixed parameters are 0, of unobserved ones NaN."""
+        xk, xp = self._x(x)
+        C, M, K = self.n_cams, self.n_poses, self.n_keys
+        cam, pose = np.empty((15 * C, 15 * C)), np.empty((M, 6, 6))
+        point = np.empty((K, 3, 3)) if self.chain == L.CHAIN_SELFCAL else None
+        s2, dof = ct.c_double(), ct.c_int64()
+        L.check(self._lib.pcs_covariance(self._h, xp, _ptr(cam), _ptr(pose), _ptr(point), ct.byref(s2), ct.byref(dof)))
+        res = dict(cam=cam, pose=pose, s2=s2.value, dof=dof.value)
+        if point is not None:
+            res["point"] = point
+        return res
+
     def lm_solve(self, x0, max_iter=100, ftol=1e-8, xtol=1e-8, gtol=1e-8, lambda0=1e-3, verbose=0):
         x0k, x0p = self._x(x0)
         opts = L.LmOptions()
