@@ -264,9 +264,10 @@ PCS_API int pcs_lm_solve(pcs_problem* p, const double* x0 /*[n_free]*/, const pc
 PCS_API int pcs_covariance(pcs_problem* p, const double* x /*[n_free] or NULL*/, double* cam, double* pose, double* point,
                            double* s2, int64_t* dof);
 
-/* Dense symmetric positive definite solve S x = b with the persistent tiled Cholesky kernel that pcs_lm_solve uses for
- * the reduced camera system (the counterpart of the LSMR solve inside scipy's TRF, optimisation_handling.py:88-98).
- * Host buffers; A is column-major [n][n], only the lower triangle is read.  *info: 0 ok, 1 not positive definite.
+/* Dense symmetric positive definite solve S x = b with the persistent tiled Cholesky kernel, the kernel every
+ * factorisation of the library uses (in pcs_lm_solve the counterpart of the LSMR solve inside scipy's TRF,
+ * optimisation_handling.py:88-98).  Host buffers; A is column-major [n][n], only the lower triangle is read.
+ * *info: 0 ok, 1 not positive definite (PCS_ERR_NUMERIC), -2 the kernel's grid barrier timed out (PCS_ERR_CUDA).
  * Exposed so that the solver kernel can be tested on its own. */
 PCS_API int pcs_spd_solve(int device, int64_t n, const double* A, const double* b, double* x /*[n]*/, int* info);
 
@@ -293,7 +294,7 @@ PCS_API int pcs_timing_get(pcs_problem* p, double* normal_kernel_ms);
 PCS_API int pcs_timing_get_all(pcs_problem* p, double* ms, int64_t capacity, int64_t* n_out);
 
 /* Number of kernels of this library launched so far for the residual / Jacobian / normal-equation evaluations of
- * this problem (cuSOLVER launches inside pcs_lm_solve are not counted).  bench.py reports the difference
+ * this problem.  bench.py reports the difference
  * over its timed region as `gpu_launches`. */
 PCS_API int pcs_launch_count(const pcs_problem* p, int64_t* n_kernels);
 

@@ -59,7 +59,7 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
         if pr.returncode != 0:
             raise RuntimeError("nvcc failed: " + " ".join(cmd) + "\n" + (out or ""))
     link = [nvcc, "-shared", "-o", str(LIB), *objs, "-gencode", "arch=compute_100a,code=sm_100a",
-            "-cudart", "static", "-lcusolver", "-Xlinker", "--no-undefined"]
+            "-cudart", "static", "-Xlinker", "--no-undefined"]
     subprocess.check_call(link)
     return LIB
 

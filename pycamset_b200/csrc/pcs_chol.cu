@@ -1,9 +1,10 @@
-// pcs_chol.cu -- dense SPD solve  S x = b  of the reduced camera system, one persistent kernel.
+// pcs_chol.cu -- dense SPD solve  S x = b, one persistent kernel: every factorisation of the library.
 //
-// Replaces cusolverDnDpotrf + cusolverDnDpotrs in the LM step (the counterpart of the LSMR solve inside scipy's TRF,
-// optimisation_handling.py:88-98).  n = 15 C is small (480 at 32 cameras, 1920 at 128): the factorisation is a chain
-// of n dependent pivots, so what matters is the latency of one block step, not throughput.  cuSOLVER spends ~240 us in
-// potrf and ~90 us in the two triangular solves at n = 480; this kernel needs one grid barrier per 32-column block step:
+// Factors the reduced camera system of the LM step (the counterpart of the LSMR solve inside scipy's TRF,
+// optimisation_handling.py:88-98), the dense self-calibration fallback and the covariance.  n = 15 C is small (480 at 32
+// cameras, 1920 at 128): the factorisation is a chain of n dependent pivots, so what matters is the latency of one block
+// step, not throughput.  A vendor potrf + potrs took ~240 + ~90 us at n = 480; this kernel needs one grid barrier per
+// 32-column block step:
 //
 //   * 32 x 32 tiles of the lower triangle, in place in global memory (L2-resident); b rides along as one more block
 //     row, so the forward substitution is part of the factorisation.
@@ -549,22 +550,26 @@ size_t chol_smem_bytes()
 
 }  // namespace
 
-// Workspace + launch geometry.  grid = 0 on return means "not usable here" (caller falls back to cuSOLVER).
+// Workspace + launch geometry.  PCS_ERR_UNSUPPORTED when the kernel cannot be co-scheduled on the device.
 int chol_prepare(int device, int64_t n, double** Ldiag, unsigned long long** bar, int* grid)
 {
-    *grid = 0;
     const int nb = (int)((n + TB - 1) / TB);
     int max_optin = 0, sms = 0, coop = 0;
     PCS_CUDA(cudaDeviceGetAttribute(&max_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
     PCS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     PCS_CUDA(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device));
     const size_t smem = chol_smem_bytes();
-    if (!coop || smem > (size_t)max_optin) return PCS_OK;
-    // monotone per (kernel, device): a later, smaller problem must not lower the opt-in of a live larger one
-    PCS_CUDA(ensure_dynamic_smem(k_chol_solve, smem));
     int per_sm = 0;
-    PCS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chol_solve, CHOL_THREADS, smem));
-    if (per_sm < 1) return PCS_OK;
+    if (coop && smem <= (size_t)max_optin) {
+        // monotone per (kernel, device): a later, smaller problem must not lower the opt-in of a live larger one
+        PCS_CUDA(ensure_dynamic_smem(k_chol_solve, smem));
+        PCS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_chol_solve, CHOL_THREADS, smem));
+    }
+    if (per_sm < 1) {
+        set_error("the Cholesky kernel cannot be co-scheduled on this device: it needs a cooperative launch and one CTA with " +
+                  std::to_string(smem) + " bytes of shared memory per SM");
+        return PCS_ERR_UNSUPPORTED;
+    }
     // work units of the widest phase: nb panel tiles + the 2 x 2 groups of the trailing tiles.  A grid wider than that only
     // makes the barrier slower (every CTA arrives on one counter)
     const int n_pairs0 = (nb + 1) / 2;
@@ -594,6 +599,17 @@ int launch_chol_solve(cudaStream_t st, int grid, int64_t n, double* A, int64_t l
     return PCS_OK;
 }
 
+// 1: a pivot was not positive; -2: a grid barrier or the back substitution's mailbox gave up waiting (the result is void)
+int chol_status(int info)
+{
+    if (info == 0) return PCS_OK;
+    if (info == -2) {
+        set_error("the Cholesky kernel's grid barrier timed out");
+        return PCS_ERR_CUDA;
+    }
+    return PCS_ERR_NUMERIC;
+}
+
 }  // namespace pcs
 
 extern "C" int pcs_spd_solve(int device, int64_t n, const double* A, const double* b, double* x, int* info)
@@ -607,7 +623,6 @@ extern "C" int pcs_spd_solve(int device, int64_t n, const double* A, const doubl
     int* dinfo = nullptr;
     int grid = 0;
     int rc = chol_prepare(device, n, &Ldiag, &bar, &grid);
-    if (rc == PCS_OK && grid == 0) { set_error("pcs_spd_solve: n too large for the persistent kernel on this device"); rc = PCS_ERR_UNSUPPORTED; }
     auto cleanup = [&]() { cudaFree(dA); cudaFree(db); cudaFree(Ldiag); cudaFree(bar); cudaFree(dinfo); };
     if (rc != PCS_OK) { cleanup(); return rc; }
     cudaError_t e = cudaMalloc((void**)&dA, (size_t)(n * n) * 8);
@@ -627,6 +642,7 @@ extern "C" int pcs_spd_solve(int device, int64_t n, const double* A, const doubl
     }
     if (info) *info = h_info;
     cleanup();
-    if (rc == PCS_OK && h_info != 0) { set_error("pcs_spd_solve: matrix is not positive definite"); rc = PCS_ERR_NUMERIC; }
+    if (rc == PCS_OK) rc = chol_status(h_info);
+    if (rc == PCS_ERR_NUMERIC) set_error("pcs_spd_solve: matrix is not positive definite");
     return rc;
 }

@@ -179,10 +179,11 @@ struct SchurPlan {
 int schur_plan_build(pcs_problem* p, int64_t nc, int64_t nl, SchurPlan* plan);
 void schur_plan_free(SchurPlan* plan);
 int launch_schur_syrk(cudaStream_t st, int sm_count, int64_t n, int64_t k, const double* Z, double* S, const SchurPlan* plan = nullptr);
-// pcs_chol.cu: dense SPD solve of the reduced camera system in one persistent kernel
+// pcs_chol.cu: dense SPD solve in one persistent kernel, every factorisation of the library
 int chol_prepare(int device, int64_t n, double** Ldiag, unsigned long long** bar, int* grid);
 int launch_chol_solve(cudaStream_t st, int grid, int64_t n, double* A, int64_t ld, double* rhs, double* Ldiag,
                       unsigned long long* bar, unsigned long long* bar_base, int* info, long long* trace = nullptr);
+int chol_status(int info);   // the kernel's info word as a pcs_status
 void p2p_free(pcs_problem* p);
 // pcs_cov.cu: covariance from the factored reduced system (S off-diagonal tiles of L, Ldiag its diagonal tiles)
 int cov_forward_substitution(cudaStream_t st, int64_t nc, const double* S, double* Ldiag, double* Xi, double* Z, int64_t np);

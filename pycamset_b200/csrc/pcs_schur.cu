@@ -2,7 +2,7 @@
 //
 // Part of the LM step that stands in for scipy's TRF / LSMR solve (optimisation_handling.py:88-98): with
 // Z = W L^-T (15 C x 6 M, dense when every camera sees every pose) the Schur complement of the pose blocks is
-// S = U + lambda D - Z Z^T.  cuBLAS DSYRK reaches a third of the FP64 pipe on this shape (n = 480, k = 12000: few
+// S = U + lambda D - Z Z^T.  A vendor DSYRK reaches a third of the FP64 pipe on this shape (n = 480, k = 12000: few
 // output tiles, long k); this kernel is shaped for it:
 //   * 96 x 96 output tiles of the lower triangle; the (tile, k) iteration space is linearised and cut into one
 //     contiguous range per SM ("stream-K"), so all SMs finish together whatever the tile count; a CTA flushes its

@@ -6,7 +6,7 @@
 //   template chain:  eliminate the pose blocks (batched 6x6 Cholesky), form the reduced camera system
 //                    S = U + lambda D_c - Z Z^T with Z = W L^-T (k_schur_syrk, pcs_schur.cu; the dense (15C x 6M) Z
 //                    and the reduced right-hand side come from k_lm_segment_Z), [all-reduce S | rhs across ranks],
-//                    dense SPD solve (k_chol_solve, pcs_chol.cu; cuSOLVER for systems too large for it),
+//                    dense SPD solve (k_chol_solve, pcs_chol.cu),
 //                    back-substitute the poses, move to the trial point and evaluate it with the full
 //                    normal-equation kernel into the second output set -- one host synchronisation per iteration;
 //   self-calibration: poses AND target points are block diagonal but coupled to each other, so one of the two sets is
@@ -15,13 +15,11 @@
 //                    (solve_points_eliminated).  Poses eliminated (otherwise): the points join the cameras in the reduced
 //                    system (15 C + 3 K unknowns: point blocks Pk, camera x point blocks Xck on the A side, pose x point
 //                    blocks Ymk next to W on the coupling side).  Problems whose dense (camera, key) / (pose, key) tables
-//                    would not fit fall back to the dense (n_free x n_free) normal matrix + cuSOLVER Cholesky with a
-//                    residual-only trial pass.
+//                    would not fit fall back to the dense (n_free x n_free) normal matrix, factored by the same
+//                    k_chol_solve, with a residual-only trial pass.
 //   The pose elimination skips the structurally zero blocks of Z (static unit list, pcs_schur.cu).
 // Marquardt scaling (lambda * diag(J^T J)) plays the role of x_scale='jac'; Nielsen's gain-ratio update
 // drives lambda.  Fixed parameters are rows / columns replaced by the identity.
-#include <cusolverDn.h>
-
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -34,7 +32,6 @@
 namespace pcs {
 
 struct LmWorkspace {
-    cusolverDnHandle_t solver = nullptr;
     int64_t nc = 0;          // order of the reduced system: 15 C (+ 3 K), rounded up to a multiple of 32 (identity rows) so that every
                              // tile of the Cholesky kernel is full and moves with 16-byte copies, whatever C and K are
     int64_t nl = 0;          // logical order 15 C (+ 3 K)
@@ -54,14 +51,12 @@ struct LmWorkspace {
     double* delta = nullptr; // [Lparams]
     double* backup = nullptr;// [Lparams]
     double* scal = nullptr;  // [8] device scalars: pred, |dx|^2, |x|^2, ginf, cost_trial, flag
-    double* work = nullptr;
-    int lwork = 0;
     int* info = nullptr;
-    // own dense SPD solve (k_chol_solve): diagonal-block factors, grid barrier counter
-    double* Ldiag = nullptr;   // [ceil(nc / 32)][32 * 32] row-major lower factors of the diagonal tiles
+    // dense SPD solve (k_chol_solve) of order nc, or n_free on the dense path: diagonal-block factors, grid barrier counter
+    double* Ldiag = nullptr;   // [ceil(n / 32)][32 * 32] row-major lower factors of the diagonal tiles
     unsigned long long* bar = nullptr;
     unsigned long long bar_base = 0;
-    int chol_grid = 0;         // co-resident CTAs of k_chol_solve (0: use cuSOLVER)
+    int chol_grid = 0;         // co-resident CTAs of k_chol_solve
     // second set of normal-equation outputs: the trial point is evaluated speculatively with the full kernel
     double* ne_alt = nullptr;
     double* ne_orig = nullptr;
@@ -75,22 +70,9 @@ struct LmWorkspace {
     double* Hd = nullptr;    // damped copy [n_free^2]
     double* rhs = nullptr;   // [n_free]
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // device time of a solve (owned by the workspace: no leak on error returns)
-    // pcs_covariance: X_I = L^-1 [nc][nc], and a Cholesky-kernel state of its own when the LM path factors with cuSOLVER
+    // pcs_covariance: X_I = L^-1 [nc][nc]
     double* cov_Xi = nullptr;
-    double* cov_Ldiag = nullptr;
-    unsigned long long* cov_bar = nullptr;
-    unsigned long long cov_bar_base = 0;
-    int cov_grid = 0;
 };
-
-#define PCS_SOLVER(call)                                                                       \
-    do {                                                                                       \
-        cusolverStatus_t s__ = (call);                                                         \
-        if (s__ != CUSOLVER_STATUS_SUCCESS) {                                                  \
-            set_error(std::string(#call) + " -> cuSOLVER status " + std::to_string((int)s__)); \
-            return PCS_ERR_CUDA;                                                               \
-        }                                                                                      \
-    } while (0)
 
 static inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
 
@@ -660,11 +642,12 @@ __global__ void k_lm_gather_readback(const double* __restrict__ scal, const int*
     if (t == 9) out[9] = *cost_lin;
 }
 
-// dense path: Hd = H + lambda diag(H), rhs = -g ; pred / norms after the solve
+// dense path: Hd = H + lambda diag(H), rhs = -g, clears the factorisation status; pred / norms after the solve
 __global__ void k_dense_damp(int64_t n, double lambda, const double* __restrict__ H, const double* __restrict__ g,
-                             double* __restrict__ Hd, double* __restrict__ rhs)
+                             double* __restrict__ Hd, double* __restrict__ rhs, int* __restrict__ info)
 {
     int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (t == 0) *info = 0;
     if (t >= n * n) return;
     const int64_t i = t / n, j = t % n;
     double v = H[t];
@@ -730,16 +713,13 @@ void lm_free(pcs_problem* p)
     if (!w) return;
     // a solve that returned early on an error may have left the problem on the second output set
     if (w->ne_alt && w->ne_orig && p->ne == w->ne_alt) swap_normal_buffers(p, w);
-    if (w->solver) cusolverDnDestroy(w->solver);
     schur_plan_free(&w->plan);
     if (w->seg_of) cudaFree(w->seg_of);
     if (w->dck) cudaFree(w->dck);
-    double* ptrs[] = {w->L, w->y, w->Z, w->red, w->delta, w->backup, w->scal, w->work, w->Hd, w->rhs, w->Ldiag, w->ne_alt,
-                      w->cov_Xi, w->cov_Ldiag};
+    double* ptrs[] = {w->L, w->y, w->Z, w->red, w->delta, w->backup, w->scal, w->Hd, w->rhs, w->Ldiag, w->ne_alt, w->cov_Xi};
     for (double* q : ptrs) if (q) cudaFree(q);
     if (w->info) cudaFree(w->info);
     if (w->bar) cudaFree(w->bar);
-    if (w->cov_bar) cudaFree(w->cov_bar);
     if (w->h_read) cudaFreeHost(w->h_read);
     if (w->d_read) cudaFree(w->d_read);
     if (w->comb) cudaFree(w->comb);
@@ -764,19 +744,15 @@ static int lm_prepare(pcs_problem* p)
     return rc;
 }
 
-// The cuSOLVER handle is created only where the library path is actually taken (the dense self-calibration fallback, a
-// reduced system too large for the persistent Cholesky kernel, or the PCS_LM_CHOL A/B switch): creating it costs tens to
-// hundreds of milliseconds per problem, more than a whole solve of a small calibration.
-static int ensure_solver(pcs_problem* p, LmWorkspace* w)
-{
-    if (w->solver) return PCS_OK;
-    PCS_SOLVER(cusolverDnCreate(&w->solver));
-    PCS_SOLVER(cusolverDnSetStream(w->solver, p->stream));
-    return PCS_OK;
-}
-
 static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
 {
+    // Solver switches for A/B runs and tests, read whenever a workspace is built: PCS_LM_SELFCAL=dense forces the dense
+    // fallback of the self-calibration chain, PCS_LM_SELFCAL=poses its pose elimination, PCS_LM_SCHUR=dense the full
+    // iteration space (identity column order) of the pose elimination.
+    const char* env_selfcal = std::getenv("PCS_LM_SELFCAL");
+    const char* env_schur = std::getenv("PCS_LM_SCHUR");
+    const bool force_dense = env_selfcal && env_selfcal[0] == 'd', force_poses = env_selfcal && env_selfcal[0] == 'p';
+    const bool dense_schur = env_schur && env_schur[0] == 'd';
     PCS_CUDA(cudaMalloc((void**)&w->delta, (size_t)p->L * 8));
     PCS_CUDA(cudaMalloc((void**)&w->backup, (size_t)p->L * 8));
     PCS_CUDA(cudaMalloc((void**)&w->scal, 8 * 8));
@@ -786,15 +762,11 @@ static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
     PCS_CUDA(cudaMemsetAsync(w->delta, 0, (size_t)p->L * 8, p->stream));
     PCS_CUDA(cudaEventCreate(&w->ev0));
     PCS_CUDA(cudaEventCreate(&w->ev1));
-    // PCS_LM_SELFCAL=dense forces the dense fallback of the self-calibration chain (A/B runs, tests)
-    static const bool force_dense = [] { const char* e = std::getenv("PCS_LM_SELFCAL"); return e && e[0] == 'd'; }();
     if (p->chain == PCS_CHAIN_TEMPLATE || (p->Pk && !force_dense)) {
         // Which block set is eliminated.  Template chain: the poses.  Self-calibration chain: poses AND points are block
         // diagonal but coupled to each other, so only one of them can go; the larger one does (3 K point unknowns against
-        // 6 M pose unknowns; PCS_LM_SELFCAL=poses forces the pose elimination for A/B runs and tests).  The point
-        // elimination is single-rank: its reduced system contains the (rank-local) poses.
-        const char* em = std::getenv("PCS_LM_SELFCAL");
-        w->pts_elim = p->chain == PCS_CHAIN_SELFCAL && p->world == 1 && 3 * (int64_t)p->K > 6 * (int64_t)p->M && !(em && em[0] == 'p');
+        // 6 M pose unknowns).  The point elimination is single-rank: its reduced system contains the (rank-local) poses.
+        w->pts_elim = p->chain == PCS_CHAIN_SELFCAL && p->world == 1 && 3 * (int64_t)p->K > 6 * (int64_t)p->M && !force_poses;
         if (w->pts_elim) {
             w->nl = 15 * (int64_t)p->C + 6 * (int64_t)p->M;       // cameras + poses
             w->np = 3 * (int64_t)p->K;                            // eliminated: point coordinates
@@ -814,18 +786,11 @@ static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
             PCS_CUDA(cudaGetLastError());
             PCS_CUDA(cudaMalloc((void**)&w->dck, (size_t)(15 * (int64_t)p->C + 3 * (int64_t)p->K) * 8));
         }
-        // block-sparse pose elimination (PCS_LM_SCHUR=dense: full iteration space, identity column order -- A/B runs, tests)
-        const char* es = std::getenv("PCS_LM_SCHUR");
-        if (!w->pts_elim && !(es && es[0] == 'd')) PCS_TRY(schur_plan_build(p, w->nc, w->nl, &w->plan));
+        // block-sparse pose elimination
+        if (!w->pts_elim && !dense_schur) PCS_TRY(schur_plan_build(p, w->nc, w->nl, &w->plan));
         w->red_doubles = w->nc * w->nc + 2 * w->nc + 1;
         PCS_CUDA(cudaMalloc((void**)&w->red, (size_t)w->red_doubles * 8));
-        // own persistent Cholesky solve (PCS_LM_CHOL=cusolver selects the library path for A/B runs)
-        const char* e = std::getenv("PCS_LM_CHOL");
-        if (!(e && e[0] == 'c')) PCS_TRY(chol_prepare(p->device, w->nc, &w->Ldiag, &w->bar, &w->chol_grid));
-        if (w->chol_grid == 0) {
-            PCS_TRY(ensure_solver(p, w));
-            PCS_SOLVER(cusolverDnDpotrf_bufferSize(w->solver, CUBLAS_FILL_MODE_LOWER, (int)w->nc, w->red, (int)w->nc, &w->lwork));
-        }
+        PCS_TRY(chol_prepare(p->device, w->nc, &w->Ldiag, &w->bar, &w->chol_grid));
         PCS_CUDA(cudaMalloc((void**)&w->ne_alt, (size_t)p->ne_doubles * 8));
         w->ne_orig = p->ne;
     } else {
@@ -835,10 +800,8 @@ static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
         w->H = p->dense;
         PCS_CUDA(cudaMalloc((void**)&w->Hd, (size_t)(n * n) * 8));
         PCS_CUDA(cudaMalloc((void**)&w->rhs, (size_t)n * 8));
-        PCS_TRY(ensure_solver(p, w));
-        PCS_SOLVER(cusolverDnDpotrf_bufferSize(w->solver, CUBLAS_FILL_MODE_LOWER, (int)n, w->Hd, (int)n, &w->lwork));
+        PCS_TRY(chol_prepare(p->device, n, &w->Ldiag, &w->bar, &w->chol_grid));
     }
-    PCS_CUDA(cudaMalloc((void**)&w->work, (size_t)std::max(w->lwork, 1) * 8));
     return PCS_OK;
 }
 
@@ -896,20 +859,12 @@ static int build_reduced(pcs_problem* p, LmWorkspace* w, double lambda)
     return PCS_OK;
 }
 
-// S = L L^T and rhs <- S^-1 rhs (the Cholesky kernel leaves the off-diagonal tiles of L in S, the diagonal ones in Ldiag)
-static int factor_solve_reduced(pcs_problem* p, LmWorkspace* w)
+// A = L L^T and rhs <- A^-1 rhs for A of order n (leading dimension ld, lower triangle read), with the workspace's
+// Cholesky-kernel state: the kernel leaves the off-diagonal tiles of L in A, the diagonal ones in Ldiag, and only ever
+// raises w->info, which must be zero on entry
+static int chol_solve(pcs_problem* p, LmWorkspace* w, int64_t n, double* A, int64_t ld, double* rhs)
 {
-    cudaStream_t st = p->stream;
-    const int64_t nc = w->nc;
-    double* Smat = w->red;
-    double* rhs = w->red + nc * nc;
-    if (w->chol_grid > 0) {
-        PCS_TRY(launch_chol_solve(st, w->chol_grid, nc, Smat, nc, rhs, w->Ldiag, w->bar, &w->bar_base, w->info));
-    } else {
-        PCS_SOLVER(cusolverDnDpotrf(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, Smat, (int)nc, w->work, w->lwork, w->info));
-        PCS_SOLVER(cusolverDnDpotrs(w->solver, CUBLAS_FILL_MODE_LOWER, (int)nc, 1, Smat, (int)nc, rhs, (int)nc, w->info));
-    }
-    return PCS_OK;
+    return launch_chol_solve(p->stream, w->chol_grid, n, A, ld, rhs, w->Ldiag, w->bar, &w->bar_base, w->info);
 }
 
 // Self-calibration chain, points eliminated (w->pts_elim): same contract as solve_template below.
@@ -919,7 +874,7 @@ static int solve_points_eliminated(pcs_problem* p, LmWorkspace* w, double lambda
     const int64_t nc = w->nc, n_cam = 15 * (int64_t)p->C;
     double* rhs = w->red + nc * nc;
     PCS_TRY(build_reduced(p, w, lambda));
-    PCS_TRY(factor_solve_reduced(p, w));
+    PCS_TRY(chol_solve(p, w, nc, w->red, nc, rhs));
     p->n_launches += 7;
     // rhs now holds [delta_c | delta_m]; the points follow from the back substitution
     PCS_CUDA(cudaMemcpyAsync(w->dck, rhs, (size_t)n_cam * 8, cudaMemcpyDeviceToDevice, st));
@@ -942,7 +897,7 @@ static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
     double* rhs = w->red + nc * nc;
     const bool selfcal = p->chain == PCS_CHAIN_SELFCAL;
     PCS_TRY(build_reduced(p, w, lambda));
-    PCS_TRY(factor_solve_reduced(p, w));
+    PCS_TRY(chol_solve(p, w, nc, w->red, nc, rhs));
     p->n_launches += 8;
     // rhs now holds delta_c
     double* dp = w->delta + 15 * (int64_t)p->C;  // pose part of the parameter-string delta is written in place
@@ -1058,19 +1013,19 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
             cost_lin = w->h_read[9];
             ginf_cam = h_scal[4];
             cost_new = h_scal[6];
-            if (h_info != 0 || h_scal[5] != 0.0) rc = PCS_ERR_NUMERIC;
+            rc = chol_status(h_info);
+            if (rc == PCS_OK && h_scal[5] != 0.0) rc = PCS_ERR_NUMERIC;
         } else {
             double *H = w->H, *g = w->H + n * n, *c = g + n;
             PCS_CUDA(cudaMemsetAsync(w->scal, 0, 8 * 8, st));
-            k_dense_damp<<<grid_for(n * n, 256), 256, 0, st>>>(n, lambda, H, g, w->Hd, w->rhs);
-            PCS_SOLVER(cusolverDnDpotrf(w->solver, CUBLAS_FILL_MODE_LOWER, (int)n, w->Hd, (int)n, w->work, w->lwork, w->info));
-            PCS_SOLVER(cusolverDnDpotrs(w->solver, CUBLAS_FILL_MODE_LOWER, (int)n, 1, w->Hd, (int)n, w->rhs, (int)n, w->info));
+            k_dense_damp<<<grid_for(n * n, 256), 256, 0, st>>>(n, lambda, H, g, w->Hd, w->rhs, w->info);
+            PCS_TRY(chol_solve(p, w, n, w->Hd, n, w->rhs));
             k_dense_delta<<<grid_for(n, 128), 128, 0, st>>>(n, lambda, w->rhs, H, g, p->free_idx, p->params, w->delta, w->scal);
             PCS_CUDA(cudaMemcpyAsync(h_scal, w->scal, 8 * 8, cudaMemcpyDeviceToHost, st));
             PCS_CUDA(cudaMemcpyAsync(&h_info, w->info, sizeof(int), cudaMemcpyDeviceToHost, st));
             PCS_CUDA(cudaMemcpyAsync(&cost_lin, c, 8, cudaMemcpyDeviceToHost, st));
             PCS_CUDA(cudaStreamSynchronize(st));
-            if (h_info != 0) rc = PCS_ERR_NUMERIC;
+            rc = chol_status(h_info);
         }
         // the template chain has already moved to the trial point: undo = old parameters + old output set
         auto undo_trial = [&]() -> int {
@@ -1185,22 +1140,6 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
     cudaStream_t st = p->stream;
     const int64_t nc = w->nc, np = w->np, n_cam = 15 * (int64_t)p->C;
     if (!w->cov_Xi) PCS_CUDA(cudaMalloc((void**)&w->cov_Xi, (size_t)(nc * nc) * 8));
-    // the factor is always the Cholesky kernel's (off-diagonal tiles of L in S, diagonal tiles in Ldiag), whichever
-    // factorisation the LM path uses
-    double* Ldiag = w->Ldiag;
-    unsigned long long* bar = w->bar;
-    unsigned long long* bar_base = &w->bar_base;
-    int grid = w->chol_grid;
-    if (grid == 0) {
-        if (!w->cov_Ldiag) {
-            PCS_TRY(chol_prepare(p->device, nc, &w->cov_Ldiag, &w->cov_bar, &w->cov_grid));
-            if (w->cov_grid == 0) {
-                set_error("pcs_covariance: the reduced system is too large for the Cholesky kernel on this device");
-                return PCS_ERR_UNSUPPORTED;
-            }
-        }
-        Ldiag = w->cov_Ldiag; bar = w->cov_bar; bar_base = &w->cov_bar_base; grid = w->cov_grid;
-    }
     if (x && p->n_free > 0) {
         PCS_TRY(ensure_pinned(p, p->n_free));
         std::memcpy(p->h_pin, x, (size_t)p->n_free * 8);
@@ -1215,9 +1154,10 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
     PCS_TRY(rc_eval);
     double* Smat = w->red;
     PCS_TRY(build_reduced(p, w, 0.0));
-    PCS_TRY(launch_chol_solve(st, grid, nc, Smat, nc, w->red + nc * nc, Ldiag, bar, bar_base, w->info));
+    // the factor: off-diagonal tiles of L in S, diagonal tiles in Ldiag
+    PCS_TRY(chol_solve(p, w, nc, Smat, nc, w->red + nc * nc));
     // X = L^-1 [I | Z] in place (Z's columns become X_b), then Sigma_red = X_I^T X_I into S (negated), Sigma_bb over L_b
-    PCS_TRY(cov_forward_substitution(st, nc, Smat, Ldiag, w->cov_Xi, w->Z, np));
+    PCS_TRY(cov_forward_substitution(st, nc, Smat, w->Ldiag, w->cov_Xi, w->Z, np));
     PCS_TRY(cov_reduced_inverse(st, p->sm_count, nc, w->cov_Xi, Smat));
     const int elim_B = w->pts_elim ? 3 : 6;
     const int n_elim = w->pts_elim ? p->K : p->M;
@@ -1237,14 +1177,11 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
     PCS_CUDA(cudaStreamSynchronize(st));
     int info = 0;
     std::memcpy(&info, h + 8, sizeof(int));
-    if (info == -2) {
-        set_error("pcs_covariance: the Cholesky kernel's grid barrier timed out");
-        return PCS_ERR_CUDA;
-    }
-    if (info != 0 || h[5] != 0.0) {
+    int rc = chol_status(info);
+    if (rc == PCS_OK && h[5] != 0.0) rc = PCS_ERR_NUMERIC;
+    if (rc == PCS_ERR_NUMERIC)
         set_error("pcs_covariance: the undamped normal equations are not positive definite (is the gauge fixed?)");
-        return PCS_ERR_NUMERIC;
-    }
+    PCS_TRY(rc);
     const int64_t d = 2 * p->N - (int64_t)h[7];
     if (dof) *dof = d;
     if (s2) *s2 = d > 0 ? h[9] / (double)d : std::nan("");

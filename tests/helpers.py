@@ -1,6 +1,8 @@
 """Shared helpers for the parity tests (oracle side only; test infrastructure)."""
 from __future__ import annotations
 
+import contextlib
+import os
 from pathlib import Path
 
 import numpy as np
@@ -34,3 +36,17 @@ def oracle_problem(g):
 def rel_err(a, b, floor=1e-12):
     a = np.asarray(a, np.float64); b = np.asarray(b, np.float64)
     return np.max(np.abs(a - b) / np.maximum(np.abs(b), floor)) if a.size else 0.0
+
+
+@contextlib.contextmanager
+def solver_env(**switches):
+    """Exactly the given PCS_LM_* solver switches inside the block (the library reads them when it builds a problem's
+    solver workspace), the caller's environment restored on exit."""
+    saved = {k: os.environ.pop(k) for k in list(os.environ) if k.startswith("PCS_LM_")}
+    os.environ.update(switches)
+    try:
+        yield
+    finally:
+        for k in switches:
+            os.environ.pop(k, None)
+        os.environ.update(saved)

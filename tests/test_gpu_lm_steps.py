@@ -10,23 +10,17 @@ built on the CPU oracle's normal equations.
   D  termination by gtol, ftol and xtol (with |x| the norm of the free vector).
 
 Each fixture is a distinct path of the solver: template chain with pose elimination (small and padded, partial masks,
-goldens, the sparse Schur plan and its dense / cuSOLVER alternatives, more cameras than the Z kernel's window with the
-chunked Cholesky); self-calibration with the points eliminated, with the poses eliminated and on the dense fallback."""
+goldens, the sparse Schur plan and its dense alternative, more cameras than the Z kernel's window with the chunked
+Cholesky); self-calibration with the points eliminated, with the poses eliminated and on the dense fallback."""
 import functools
-import json
-import os
-import subprocess
-import sys
-import tempfile
-from pathlib import Path
 
 import numpy as np
 import pytest
 
 from tests import lm_reference as R
+from tests.helpers import solver_env
 
 pytestmark = pytest.mark.gpu
-ROOT = Path(__file__).resolve().parent.parent
 LAMBDAS = (1e-6, 1e-3, 1.0, 1e2)
 
 
@@ -40,59 +34,24 @@ def model(name, path="block"):
     return fixture(name).model(path)
 
 
-_CHILD = """
-import sys, json, numpy as np
-sys.path.insert(0, {root!r})
-from tests import lm_reference as R
-fx = R.FIXTURES[{name!r}]()
-runs = json.loads({runs!r})
-out = {{}}
-with fx.problem() as p:
-    for i, r in enumerate(runs):
-        p.set_param_string(fx.params0)
-        x, st = p.lm_solve(fx.x0, **r)
-        out["x%d" % i] = x
-        out["p%d" % i] = p.get_param_string()
-        out["s%d" % i] = np.array([json.dumps(st)])
-np.savez({path!r}, **out)
-"""
-
-
 def device_runs(name, runs, env=None):
     """[(x, stats, parameter string)] of lm_solve(x0, **run) for each run, every run from the fixture's start.
-    env: solver switches.  PCS_LM_SCHUR / PCS_LM_CHOL are read when the solver workspace is built (in-process);
-    PCS_LM_SELFCAL=dense is read once per process, so those runs go to a child interpreter."""
+    env: solver switches (PCS_LM_*), read when the problem's solver workspace is built."""
     env = env or {}
     fx = fixture(name)
-    if "PCS_LM_SELFCAL" in env:
-        with tempfile.TemporaryDirectory() as d:
-            path = os.path.join(d, "out.npz")
-            e = {k: v for k, v in os.environ.items() if not k.startswith("PCS_LM_")} | env
-            pr = subprocess.run([sys.executable, "-c", _CHILD.format(root=str(ROOT), name=name, runs=json.dumps(runs), path=path)],
-                                capture_output=True, text=True, env=e, timeout=1200)
-            assert pr.returncode == 0, pr.stderr[-3000:]
-            z = np.load(path)
-            return [(z[f"x{i}"], json.loads(str(z[f"s{i}"][0])), z[f"p{i}"]) for i in range(len(runs))]
-    saved = {k: os.environ.pop(k) for k in list(os.environ) if k.startswith("PCS_LM_")}
-    os.environ.update(env)
-    try:
-        out = []
-        with fx.problem() as p:
-            if name == "ring32_template":
-                frac = p.lm_schur_fraction()
-                if "PCS_LM_SCHUR" in env:
-                    assert frac == 1.0
-                else:
-                    assert 0.2 < frac < 0.85, frac
-            for r in runs:
-                p.set_param_string(fx.params0)
-                x, st = p.lm_solve(fx.x0, **r)
-                out.append((x, st, p.get_param_string()))
-        return out
-    finally:
-        for k in env:
-            os.environ.pop(k, None)
-        os.environ.update(saved)
+    out = []
+    with solver_env(**env), fx.problem() as p:
+        if name == "ring32_template":
+            frac = p.lm_schur_fraction()
+            if "PCS_LM_SCHUR" in env:
+                assert frac == 1.0
+            else:
+                assert 0.2 < frac < 0.85, frac
+        for r in runs:
+            p.set_param_string(fx.params0)
+            x, st = p.lm_solve(fx.x0, **r)
+            out.append((x, st, p.get_param_string()))
+    return out
 
 
 def _path_label(name, env):
@@ -107,7 +66,6 @@ ONE_STEP = [
     ("ccube_template", {}, LAMBDAS),
     ("ring32_template", {}, LAMBDAS),
     ("ring32_template", {"PCS_LM_SCHUR": "dense"}, (1e-3, 1.0)),
-    ("ring32_template", {"PCS_LM_CHOL": "cusolver"}, (1e-3, 1.0)),
     ("dome128_template", {}, (1e-3, 1.0)),
     ("rig4_selfcal_point_masks", {}, (1e-3, 1.0, 1e2)),
     ("ccube_selfcal", {}, (1e-3, 1.0)),

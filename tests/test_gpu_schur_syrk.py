@@ -6,6 +6,8 @@ fewer work units than SMs, and the bench shape (480 x 12000).  Tolerance: |dS| <
 import numpy as np
 import pytest
 
+from tests.helpers import solver_env
+
 pytestmark = pytest.mark.gpu
 
 
@@ -31,7 +33,6 @@ def test_syrk_matches_numpy(n, k):
 
 def _ring_lm(max_iter, dense):
     """LM iterates of a 32-camera ring (every pose seen by about half of the cameras) with / without the sparsity plan."""
-    import os
     from pycamset_b200 import synthetic as syn
     from pycamset_b200.problem import BundleProblem
     rig = syn.make_rig(32, 300, distortion=True, seed=3, detect_prob=0.9)
@@ -39,19 +40,12 @@ def _ring_lm(max_iter, dense):
     params = rig.param_string(intr, extr, poses)
     unfixed = np.ones(params.shape[0], bool)
     unfixed[15 * 32:15 * 32 + 6] = False
-    old = os.environ.pop("PCS_LM_SCHUR", None)
-    if dense:
-        os.environ["PCS_LM_SCHUR"] = "dense"   # read when the solver workspace is built
-    try:
-        with BundleProblem(0, rig.cam.numpy(), rig.pose.numpy(), rig.key.numpy(), rig.uv.numpy(), 32, 300, 81, template=rig.template,
-                           unfixed=unfixed) as p:
-            p.set_param_string(params)
-            frac = p.lm_schur_fraction()
-            x, st = p.lm_solve(params[unfixed], max_iter=max_iter, ftol=0, xtol=0, gtol=0)
-    finally:
-        os.environ.pop("PCS_LM_SCHUR", None)
-        if old is not None:
-            os.environ["PCS_LM_SCHUR"] = old
+    with solver_env(**({"PCS_LM_SCHUR": "dense"} if dense else {})), \
+            BundleProblem(0, rig.cam.numpy(), rig.pose.numpy(), rig.key.numpy(), rig.uv.numpy(), 32, 300, 81, template=rig.template,
+                          unfixed=unfixed) as p:
+        p.set_param_string(params)
+        frac = p.lm_schur_fraction()
+        x, st = p.lm_solve(params[unfixed], max_iter=max_iter, ftol=0, xtol=0, gtol=0)
     return frac, x, st
 
 

@@ -5,21 +5,15 @@ free_point; BASELINE.json config 3, standard_bundle_handler.py:129-226).
     the corresponding block of the oracle's dense J^T J / J^T r with no parameter fixed (tolerance 1e-9 sqrt(d_a d_b));
   * the device LM on the block path, in both elimination orders (points eliminated, cameras + poses in the reduced system
     -- the library's choice when 3 K > 6 M; or poses eliminated, cameras + points in the reduced system), own SYRK +
-    Cholesky kernels, against the dense n_free x n_free path (cuSOLVER), which stays as the comparator: same cost trajectory."""
-import os
-import subprocess
-import sys
-from pathlib import Path
-
+    Cholesky kernels, against the dense n_free x n_free path, which stays as the comparator: same cost trajectory."""
 import numpy as np
 import pytest
 
 from oracle import oracle as orc
-from tests.helpers import available, load_case, oracle_problem
+from tests.helpers import available, load_case, oracle_problem, solver_env
 
 pytestmark = pytest.mark.gpu
 CASES = available(["ring4_selfcal", "ring5_fixedcam_selfcal", "ccube_selfcal"])
-ROOT = Path(__file__).resolve().parent.parent
 
 
 def _problem(g):
@@ -64,47 +58,27 @@ def test_selfcal_blocks_against_the_oracle(case):
         assert not JtJ[np.ix_(cam_idx[c], pose_idx[m])].any()
 
 
-_CHILD = """
-import sys, json, numpy as np
-sys.path.insert(0, {root!r})
-from tests.helpers import load_case
-from pycamset_b200.problem import BundleProblem
-g = load_case({case!r})
-dd = g["dd"]
-with BundleProblem(1, dd[:, 0], dd[:, 1], dd[:, 2], dd[:, 3:5], int(g["n_cams"]), int(g["n_poses"]), g["template"].shape[0],
-                   unfixed=g["unfixed"]) as p:
-    p.set_param_string(g["param0"])
+def _lm_runs(case, mode):
+    """Four LM solves (max_iter 1, 2, 5, 100) from the golden start on a fresh problem.  mode: None = the library's choice
+    (the larger of the pose / point block sets is eliminated), "poses" = pose elimination forced (cameras + points in the
+    reduced system), "dense" = the dense n_free x n_free comparator."""
+    g = load_case(case)
     out = []
-    for it in (1, 2, 5, 100):
-        p.set_param_string(g["param0"])
-        x, st = p.lm_solve(g["x"], max_iter=it, ftol=1e-12, xtol=1e-12, gtol=1e-12)
-        r = p.residual(x)
-        out.append(dict(it=st["iterations"], cost=st["cost_final"], true_cost=0.5 * float(r @ r), seconds=st["seconds"],
-                        px=float(np.mean(np.linalg.norm(r.reshape(-1, 2), axis=1)))))
-print("RESULT" + json.dumps(out))
-"""
-
-
-def _run_child(case, mode):
-    """mode: None = the library's choice (the larger of the pose / point block sets is eliminated), "poses" = pose
-    elimination forced (cameras + points in the reduced system), "dense" = the dense n_free x n_free comparator."""
-    import json
-    env = dict(os.environ)
-    env.pop("PCS_LM_SELFCAL", None)
-    if mode:
-        env["PCS_LM_SELFCAL"] = mode
-    pr = subprocess.run([sys.executable, "-c", _CHILD.format(root=str(ROOT), case=case)], capture_output=True, text=True, env=env,
-                        timeout=600)
-    assert pr.returncode == 0, pr.stderr[-2000:]
-    return json.loads([l for l in pr.stdout.splitlines() if l.startswith("RESULT")][-1][6:])
+    with solver_env(**({"PCS_LM_SELFCAL": mode} if mode else {})), _problem(g) as p:
+        for it in (1, 2, 5, 100):
+            p.set_param_string(g["param0"])
+            x, st = p.lm_solve(g["x"], max_iter=it, ftol=1e-12, xtol=1e-12, gtol=1e-12)
+            r = p.residual(x)
+            out.append(dict(it=st["iterations"], cost=st["cost_final"], true_cost=0.5 * float(r @ r), seconds=st["seconds"],
+                            px=float(np.mean(np.linalg.norm(r.reshape(-1, 2), axis=1)))))
+    return out
 
 
 @pytest.mark.parametrize("case", CASES)
 def test_selfcal_block_lm_matches_the_dense_path(case):
-    """The library picks the path once per process (PCS_LM_SELFCAL), so each arm runs in its own interpreter."""
-    dns = _run_child(case, "dense")
+    dns = _lm_runs(case, "dense")
     for mode in (None, "poses"):             # both elimination orders of the block path: the same Newton systems, solved differently
-        blk = _run_child(case, mode)
+        blk = _lm_runs(case, mode)
         for b, d in zip(blk[:3], dns[:3]):   # the first iterations: same linear systems, solved two ways
             assert b["it"] == d["it"]
             assert abs(b["cost"] - d["cost"]) <= 1e-8 * d["cost"], (mode, b, d)
