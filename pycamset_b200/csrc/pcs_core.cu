@@ -1183,6 +1183,10 @@ int pcs_set_allreduce(pcs_problem* p, pcs_allreduce_fn fn, void* user, int rank,
 {
     PCS_REQUIRE(p, "NULL argument");
     PCS_REQUIRE(world_size >= 1 && rank >= 0 && rank < world_size, "rank / world_size out of range");
+    if (world_size != p->world) {   // the LM workspace is laid out for one world size (its path, its all-reduce buffers)
+        PCS_CUDA(cudaSetDevice(p->device));
+        lm_free(p);
+    }
     p->allreduce = world_size > 1 ? fn : nullptr;
     p->allreduce_user = user;
     p->rank = rank;

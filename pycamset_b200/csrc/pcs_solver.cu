@@ -2,21 +2,21 @@
 //
 // Replaces scipy.optimize.least_squares (TRF + LSMR, x_scale='jac') as driven by run_bundle_adjustment
 // (optimisation_handling.py:52-117).  The reference never forms J^T J; here the fused kernel delivers the
-// block normal equations and each LM step is
-//   template chain:  eliminate the pose blocks (batched 6x6 Cholesky), form the reduced camera system
-//                    S = U + lambda D_c - Z Z^T with Z = W L^-T (k_schur_syrk, pcs_schur.cu; the dense (15C x 6M) Z
-//                    and the reduced right-hand side come from k_lm_segment_Z), [all-reduce S | rhs across ranks],
-//                    dense SPD solve (k_chol_solve, pcs_chol.cu),
-//                    back-substitute the poses, move to the trial point and evaluate it with the full
-//                    normal-equation kernel into the second output set -- one host synchronisation per iteration;
+// block normal equations and each LM step (solve_step) eliminates one set of B x B diagonal blocks (BlockSet: the poses,
+// B = 6, or the target points, B = 3; lm_path decides which):
+//   factor the damped blocks (k_lm_block_factor<B>), form the reduced system over the cameras (+ the second block set of
+//   the self-calibration chain) S = A + lambda D - Z Z^T with Z = (coupling) L_b^-T (k_lm_init_reduced<B>, the Z kernels,
+//   k_schur_syrk in pcs_schur.cu), [all-reduce S | rhs across ranks], dense SPD solve (k_chol_solve, pcs_chol.cu),
+//   back-substitute the eliminated blocks (k_lm_block_back<B>), move to the trial point and evaluate it with the full
+//   normal-equation kernel into the second output set -- one host synchronisation per iteration.
+//   template chain:  the poses are eliminated, the reduced system is over the cameras (15 C).
 //   self-calibration: poses AND target points are block diagonal but coupled to each other, so one of the two sets is
-//                    eliminated -- the larger one.  Points eliminated (3 K > 6 M, single rank): 3 x 3 Cholesky per point,
-//                    reduced system over cameras + poses [[U, .], [W^T, V]] - Z Z^T with Z = [Xck; Ymk] L_k^-T
-//                    (solve_points_eliminated).  Poses eliminated (otherwise): the points join the cameras in the reduced
-//                    system (15 C + 3 K unknowns: point blocks Pk, camera x point blocks Xck on the A side, pose x point
-//                    blocks Ymk next to W on the coupling side).  Problems whose dense (camera, key) / (pose, key) tables
-//                    would not fit fall back to the dense (n_free x n_free) normal matrix, factored by the same
-//                    k_chol_solve, with a residual-only trial pass.
+//                    eliminated -- the larger one.  Points eliminated (3 K > 6 M, single rank): reduced system over
+//                    cameras + poses [[U, .], [W^T, V]] - Z Z^T with Z = [Xck; Ymk] L_k^-T.  Poses eliminated
+//                    (otherwise): the points join the cameras in the reduced system (15 C + 3 K unknowns: point blocks
+//                    Pk, camera x point blocks Xck on the A side, pose x point blocks Ymk next to W on the coupling side).
+//                    Problems whose dense (camera, key) / (pose, key) tables would not fit fall back to the dense
+//                    (n_free x n_free) normal matrix, factored by the same k_chol_solve, with a residual-only trial pass.
 //   The pose elimination skips the structurally zero blocks of Z (static unit list, pcs_schur.cu).
 // Marquardt scaling (lambda * diag(J^T J)) plays the role of x_scale='jac'; Nielsen's gain-ratio update
 // drives lambda.  Fixed parameters are rows / columns replaced by the identity.
@@ -31,21 +31,37 @@
 
 namespace pcs {
 
+// A set of B x B diagonal blocks of the normal equations: the poses (B = 6) or the target points (B = 3).  block_set()
+// builds it from the problem whenever it is used, because the normal-equation outputs alternate between two buffers
+// (swap_normal_buffers).
+struct BlockSet {
+    int B = 0;                       // 6: poses, 3: target points, 0: no set
+    int n = 0;                       // number of blocks
+    int64_t off = 0;                 // first parameter of the set in the parameter string
+    const double* blk = nullptr;     // [n][B][B] V / Pk
+    const double* g = nullptr;       // [n][B]    gp / gk
+    const uint8_t* mask = nullptr;   // [n] free bits
+    const int32_t* slot = nullptr;   // [n] column slot of block b in Z (pose elimination with a Schur plan), nullptr = b
+};
+
+// The LM path, fixed when the workspace is built (lm_path): the eliminated block set (elim_B = 6: poses, 3: target
+// points, 0: none -- the dense self-calibration fallback) and the second block set that joins the cameras in the reduced
+// system (red_B = 3: the points, 6: the poses, 0: none -- template chain).
+struct LmPath {
+    int elim_B = 0, red_B = 0;
+};
+
 struct LmWorkspace {
-    int64_t nc = 0;          // order of the reduced system: 15 C (+ 3 K), rounded up to a multiple of 32 (identity rows) so that every
-                             // tile of the Cholesky kernel is full and moves with 16-byte copies, whatever C and K are
-    int64_t nl = 0;          // logical order 15 C (+ 3 K)
-    int64_t np = 0;          // 6 M
-    double* L = nullptr;     // [M][36] lower Cholesky factors of damped V
-    double* y = nullptr;     // [M][6]  L^-1 b_p
-    double* Z = nullptr;     // [np][nc] column-major (nc rows): W L^-T scattered by (camera, pose)
+    LmPath path;
+    int64_t nc = 0;          // order of the reduced system nl, rounded up to a multiple of 32 (identity rows) so that every
+                             // tile of the Cholesky kernel is full and moves with 16-byte copies, whatever C, M and K are
+    int64_t nl = 0;          // logical order: 15 C + the second set's unknowns (3 K, 6 M or none)
+    int64_t np = 0;          // eliminated unknowns: 6 M or 3 K
+    double* L = nullptr;     // [n_elim][B * B] lower Cholesky factors of the damped eliminated blocks
+    double* y = nullptr;     // [n_elim][B]     L_b^-1 (-g_b)
+    double* Z = nullptr;     // [np][nc] column-major (nc rows): coupling L_b^-T
     SchurPlan plan;          // static block sparsity of Z: pose column order + non-zero (tile, slab) units (pcs_schur.cu)
-    // self-calibration chain with more point than pose unknowns (3 K > 6 M): the POINTS are eliminated (3 x 3 blocks) and
-    // the reduced system is over cameras + poses (15 C + 6 M) instead of cameras + points -- 162 instead of 1503 unknowns
-    // on the reference's ccube fixture.  L / y then hold the point factors [K][9] / [K][3], Z is [3 K][nc].
-    bool pts_elim = false;
-    int32_t* seg_of = nullptr;   // [C][M] segment of (camera, pose) or -1 (placement of the W blocks in the reduced system)
-    double* dck = nullptr;       // [15 C + 3 K] camera + point part of the step, in the layout k_lm_assemble_delta reads
+    int32_t* seg_of = nullptr;   // poses in the reduced system: [C][M] segment of (camera, pose) or -1 (placement of W)
     double* red = nullptr;   // [S nc*nc | rhs nc | gc nc | cost 1]  (all-reduce unit)
     int64_t red_doubles = 0;
     double* delta = nullptr; // [Lparams]
@@ -63,7 +79,6 @@ struct LmWorkspace {
     // one pinned read-back per iteration: scal[8] | info | cost of the linearisation point (gathered on the device)
     double* h_read = nullptr;   // pinned [10]
     double* d_read = nullptr;   // [10]
-    int comb_cap = 0;
     double* comb = nullptr;     // [5 + world] multi-rank: the step scalars of all ranks in ONE sum all-reduce (see k_lm_pack_scalars)
     // dense path
     double* H = nullptr;     // [n_free^2 + n_free + 1] = JtJ | Jtr | cost  (aliases p->dense)
@@ -76,32 +91,32 @@ struct LmWorkspace {
 
 static inline int grid_for(int64_t n, int block) { return (int)((n + block - 1) / block); }
 
-// --------------------------------------------------------------------------------------------
-// pose elimination: one thread per pose
-// --------------------------------------------------------------------------------------------
-__global__ void k_lm_pose_factor(int M, double lambda, const double* __restrict__ V, const double* __restrict__ gp,
-                                 const uint8_t* __restrict__ pose_mask, double* __restrict__ Lout, double* __restrict__ yout,
-                                 double* __restrict__ scal)
+// per block (one thread each): Cholesky of the damped, masked B x B block, y = L^-1 (-g); fixed / unobserved coordinates
+// are identity rows
+template <int B>
+__global__ void k_lm_block_factor(int n, double lambda, const double* __restrict__ blk, const double* __restrict__ g,
+                                  const uint8_t* __restrict__ blk_mask, double* __restrict__ Lout, double* __restrict__ yout,
+                                  double* __restrict__ scal)
 {
     int m = blockIdx.x * blockDim.x + threadIdx.x;
-    if (m >= M) return;
-    const unsigned mask = pose_mask[m];
-    double A[6][6], b[6];
+    if (m >= n) return;
+    const unsigned mask = blk_mask[m];
+    double A[B][B], b[B];
 #pragma unroll
-    for (int i = 0; i < 6; ++i) {
+    for (int i = 0; i < B; ++i) {
         const bool fi = mask & (1u << i);
-        b[i] = fi ? -gp[(int64_t)m * 6 + i] : 0.0;
+        b[i] = fi ? -g[(int64_t)m * B + i] : 0.0;
 #pragma unroll
-        for (int j = 0; j < 6; ++j) {
+        for (int j = 0; j < B; ++j) {
             const bool fj = mask & (1u << j);
-            double v = (fi && fj) ? V[(int64_t)m * 36 + i * 6 + j] : 0.0;
+            double v = (fi && fj) ? blk[(int64_t)m * (B * B) + i * B + j] : 0.0;
             if (i == j) v = (fi && v > 0.0) ? v + lambda * v : 1.0;  // fixed or unobserved: identity row
             A[i][j] = v;
         }
     }
     bool ok = true;
 #pragma unroll
-    for (int j = 0; j < 6; ++j) {
+    for (int j = 0; j < B; ++j) {
         double d = A[j][j];
 #pragma unroll
         for (int k = 0; k < j; ++k) d -= A[j][k] * A[j][k];
@@ -110,7 +125,7 @@ __global__ void k_lm_pose_factor(int M, double lambda, const double* __restrict_
         A[j][j] = d;
         const double inv = 1.0 / d;
 #pragma unroll
-        for (int i = j + 1; i < 6; ++i) {
+        for (int i = j + 1; i < B; ++i) {
             double s = A[i][j];
 #pragma unroll
             for (int k = 0; k < j; ++k) s -= A[i][k] * A[j][k];
@@ -120,17 +135,34 @@ __global__ void k_lm_pose_factor(int M, double lambda, const double* __restrict_
     if (!ok) scal[5] = 1.0;
     // y = L^-1 b
 #pragma unroll
-    for (int i = 0; i < 6; ++i) {
+    for (int i = 0; i < B; ++i) {
         double s = b[i];
 #pragma unroll
         for (int k = 0; k < i; ++k) s -= A[i][k] * b[k];
         b[i] = s / A[i][i];
     }
 #pragma unroll
-    for (int i = 0; i < 6; ++i) {
-        yout[(int64_t)m * 6 + i] = b[i];
+    for (int i = 0; i < B; ++i) {
+        yout[(int64_t)m * B + i] = b[i];
 #pragma unroll
-        for (int j = 0; j < 6; ++j) Lout[(int64_t)m * 36 + i * 6 + j] = (j <= i) ? A[i][j] : 0.0;
+        for (int j = 0; j < B; ++j) Lout[(int64_t)m * (B * B) + i * B + j] = (j <= i) ? A[i][j] : 0.0;
+    }
+}
+
+// One row of a coupling block times L_b^-T: z = x L_b^-T (forward substitution L_b z^T = x^T; x reads as zero unless
+// row_free, and so does every entry whose bit is clear in `live`), and dot += z . y_b -- a row of Z and its share of the
+// reduced right-hand side.  Lb = the factor of block b, y = [n][B] (all blocks)
+template <int B>
+__device__ __forceinline__ void tri_row(const double* x, bool row_free, unsigned live, const double* Lb, const double* y, int b,
+                                        double (&z)[B], double& dot)
+{
+#pragma unroll
+    for (int i = 0; i < B; ++i) {
+        double v = (row_free && (live & (1u << i))) ? x[i] : 0.0;
+#pragma unroll
+        for (int k = 0; k < i; ++k) v -= Lb[i * B + k] * z[k];
+        z[i] = v / Lb[i * B + i];
+        dot = fma(z[i], y[(int64_t)b * B + i], dot);
     }
 }
 
@@ -158,17 +190,8 @@ k_lm_segment_Z(int64_t S, int64_t nc, const int32_t* __restrict__ seg_cam, const
         const int c = seg_cam[s], m = seg_pose[s];
         const bool row_free = cam_mask[c] & (1u << a);
         const unsigned pm = pose_mask[m];
-        const double* Lm = L + (int64_t)m * 36;
         double z[6], dot = 0.0;
-#pragma unroll
-        for (int i = 0; i < 6; ++i) {
-            double w = (row_free && (pm & (1u << i))) ? W[s * 90 + a * 6 + i] : 0.0;
-#pragma unroll
-            for (int k = 0; k < i; ++k) w -= Lm[i * 6 + k] * z[k];
-            z[i] = w / Lm[i * 6 + i];
-            dot = fma(z[i], y[(int64_t)m * 6 + i], dot);
-        }
-#pragma unroll
+        tri_row<6>(W + s * 90 + a * 6, row_free, pm, L + (int64_t)m * 36, y, m, z, dot);
         const int64_t col0 = 6 * (int64_t)(pose_slot ? pose_slot[m] : m);
 #pragma unroll
         for (int i = 0; i < 6; ++i) Z[(col0 + i) * nc + (int64_t)c * 15 + a] = z[i];
@@ -185,15 +208,18 @@ k_lm_segment_Z(int64_t S, int64_t nc, const int32_t* __restrict__ seg_cam, const
     }
 }
 
-// S = [[U + lambda D, .], [Xck^T, Pk + lambda D]] (lower triangle; cameras first, then -- self-calibration chain -- the
-// target points), masked, every other entry zero (each entry of S is written exactly once: no memset); rhs = -g masked,
-// g copy (for the convergence test); also clears the step scalars and the factorisation status.
-__global__ void k_lm_init_reduced(int C, int K, int64_t nc, int64_t nl, double lambda, const double* __restrict__ U, const double* __restrict__ gc,
-                                  const double* __restrict__ cost, const uint16_t* __restrict__ cam_mask,
-                                  const double* __restrict__ Pk, const double* __restrict__ gk, const double* __restrict__ Xck,
-                                  const uint8_t* __restrict__ key_mask, double* __restrict__ Smat,
-                                  double* __restrict__ rhs, double* __restrict__ gcopy, double* __restrict__ cost_out,
-                                  double* __restrict__ scal, int* __restrict__ info)
+// S = [[U + lambda D, .], [X^T, P + lambda D]] (lower triangle; cameras first, then -- self-calibration chain -- the
+// second block set P of n B x B blocks: the target points (B = 3, coupling X = Xck) or the poses (B = 6, coupling X = the
+// W blocks placed through seg_of)), masked, every other entry zero (each entry of S is written exactly once: no memset);
+// rhs = -g masked, g copy (for the convergence test); also clears the step scalars and the factorisation status.
+// Template chain: no second set (nl = 15 C), either instantiation.
+template <int B>
+__global__ void k_lm_init_reduced(int C, int n, int64_t nc, int64_t nl, double lambda, const double* __restrict__ U,
+                                  const double* __restrict__ gc, const double* __restrict__ cost, const uint16_t* __restrict__ cam_mask,
+                                  const double* __restrict__ P, const double* __restrict__ gP, const uint8_t* __restrict__ P_mask,
+                                  const double* __restrict__ Xck, const double* __restrict__ W, const int32_t* __restrict__ seg_of,
+                                  double* __restrict__ Smat, double* __restrict__ rhs, double* __restrict__ gcopy,
+                                  double* __restrict__ cost_out, double* __restrict__ scal, int* __restrict__ info)
 {
     const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (t < 8) scal[t] = 0.0;
@@ -219,21 +245,26 @@ __global__ void k_lm_init_reduced(int C, int K, int64_t nc, int64_t nl, double l
         }
     } else if (row >= n_cam && col >= n_cam) {
         const int64_t jr = row - n_cam, jc = col - n_cam;
-        const int k = (int)(jr / 3), a = (int)(jr % 3), kb = (int)(jc / 3), b = (int)(jc % 3);
+        const int k = (int)(jr / B), a = (int)(jr % B), kb = (int)(jc / B), b = (int)(jc % B);
         if (k == kb) {
-            const unsigned mask = key_mask[k];
+            const unsigned mask = P_mask[k];
             const bool fa = mask & (1u << a), fb = mask & (1u << b);
-            v = (fa && fb) ? Pk[(int64_t)k * 9 + a * 3 + b] : 0.0;
+            v = (fa && fb) ? P[(int64_t)k * (B * B) + a * B + b] : 0.0;
             if (a == b) {
                 v = fa ? v + lambda * v : 0.0;
-                rhs[row] = fa ? -gk[jr] : 0.0;
-                gcopy[row] = fa ? gk[jr] : 0.0;
+                rhs[row] = fa ? -gP[jr] : 0.0;
+                gcopy[row] = fa ? gP[jr] : 0.0;
             }
         }
-    } else if (row >= n_cam) {   // point row, camera column: Xck[c][k][i][a]
+    } else if (row >= n_cam) {   // second-set row (block k, coordinate a), camera column (camera c, coordinate i)
         const int64_t jr = row - n_cam;
-        const int k = (int)(jr / 3), a = (int)(jr % 3), c = (int)(col / 15), i = (int)(col % 15);
-        if ((key_mask[k] & (1u << a)) && (cam_mask[c] & (1u << i))) v = Xck[(((int64_t)c * K + k) * 15 + i) * 3 + a];
+        const int k = (int)(jr / B), a = (int)(jr % B), c = (int)(col / 15), i = (int)(col % 15);
+        if (B == 3) {            // points: Xck[c][k][i][a]
+            if ((P_mask[k] & (1u << a)) && (cam_mask[c] & (1u << i))) v = Xck[(((int64_t)c * n + k) * 15 + i) * 3 + a];
+        } else {                 // poses: W_s[i][a] of the segment s of (camera c, pose k)
+            const int32_t s = seg_of[(int64_t)c * n + k];
+            if (s >= 0 && (P_mask[k] & (1u << a)) && (cam_mask[c] & (1u << i))) v = W[(int64_t)s * 90 + i * 6 + a];
+        }
     }
     Smat[t] = v;
 }
@@ -259,16 +290,8 @@ k_lm_point_Z(int M, int K, int64_t nc, int64_t row0, const double* __restrict__ 
     if (!any) return;
     const bool row_free = key_mask[k] & (1u << a);
     const unsigned pm = pose_mask[m];
-    const double* Lm = L + (int64_t)m * 36;
     double z[6], dot = 0.0;
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-        double v = (row_free && (pm & (1u << i))) ? w[i] : 0.0;
-#pragma unroll
-        for (int q = 0; q < i; ++q) v -= Lm[i * 6 + q] * z[q];
-        z[i] = v / Lm[i * 6 + i];
-        dot = fma(z[i], y[(int64_t)m * 6 + i], dot);
-    }
+    tri_row<6>(w, row_free, pm, L + (int64_t)m * 36, y, m, z, dot);
     const int64_t row = row0 + 3 * (int64_t)k + a;
     const int64_t col0 = 6 * (int64_t)(pose_slot ? pose_slot[m] : m);
 #pragma unroll
@@ -281,113 +304,6 @@ __global__ void k_seg_of(int64_t S, int M, const int32_t* __restrict__ seg_cam, 
 {
     const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (s < S) seg_of[(int64_t)seg_cam[s] * M + seg_pose[s]] = (int32_t)s;
-}
-
-// per point: Cholesky of the damped, masked 3 x 3 block, y = L^-1 (-g); fixed / unobserved coordinates are identity rows
-__global__ void k_lm_point_factor(int K, double lambda, const double* __restrict__ Pk, const double* __restrict__ gk,
-                                  const uint8_t* __restrict__ key_mask, double* __restrict__ Lout, double* __restrict__ yout,
-                                  double* __restrict__ scal)
-{
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= K) return;
-    const unsigned mask = key_mask[k];
-    double A[3][3], b[3];
-#pragma unroll
-    for (int i = 0; i < 3; ++i) {
-        const bool fi = mask & (1u << i);
-        b[i] = fi ? -gk[3 * (int64_t)k + i] : 0.0;
-#pragma unroll
-        for (int j = 0; j < 3; ++j) {
-            const bool fj = mask & (1u << j);
-            double v = (fi && fj) ? Pk[(int64_t)k * 9 + i * 3 + j] : 0.0;
-            if (i == j) v = (fi && v > 0.0) ? v + lambda * v : 1.0;
-            A[i][j] = v;
-        }
-    }
-    bool ok = true;
-#pragma unroll
-    for (int j = 0; j < 3; ++j) {
-        double d = A[j][j];
-#pragma unroll
-        for (int q = 0; q < j; ++q) d -= A[j][q] * A[j][q];
-        if (!(d > 0.0)) { ok = false; d = 1.0; }
-        d = sqrt(d);
-        A[j][j] = d;
-        const double inv = 1.0 / d;
-#pragma unroll
-        for (int i = j + 1; i < 3; ++i) {
-            double s = A[i][j];
-#pragma unroll
-            for (int q = 0; q < j; ++q) s -= A[i][q] * A[j][q];
-            A[i][j] = s * inv;
-        }
-    }
-    if (!ok) scal[5] = 1.0;
-#pragma unroll
-    for (int i = 0; i < 3; ++i) {
-        double s = b[i];
-#pragma unroll
-        for (int q = 0; q < i; ++q) s -= A[i][q] * b[q];
-        b[i] = s / A[i][i];
-    }
-#pragma unroll
-    for (int i = 0; i < 3; ++i) {
-        yout[3 * (int64_t)k + i] = b[i];
-#pragma unroll
-        for (int j = 0; j < 3; ++j) Lout[(int64_t)k * 9 + i * 3 + j] = (j <= i) ? A[i][j] : 0.0;
-    }
-}
-
-// S = [[U + lambda D, .], [W^T, V + lambda D]] over cameras + poses (lower triangle, every entry written once), masked;
-// rhs = -g, g copy; clears the step scalars and the factorisation status (as k_lm_init_reduced does)
-__global__ void k_lm_init_reduced_cp(int C, int M, int64_t nc, int64_t nl, double lambda, const double* __restrict__ U,
-                                     const double* __restrict__ gc, const double* __restrict__ V, const double* __restrict__ gp,
-                                     const double* __restrict__ W, const int32_t* __restrict__ seg_of, const double* __restrict__ cost,
-                                     const uint16_t* __restrict__ cam_mask, const uint8_t* __restrict__ pose_mask,
-                                     double* __restrict__ Smat, double* __restrict__ rhs, double* __restrict__ gcopy,
-                                     double* __restrict__ cost_out, double* __restrict__ scal, int* __restrict__ info)
-{
-    const int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (t < 8) scal[t] = 0.0;
-    if (t == 8) { *info = 0; *cost_out = *cost; }
-    if (t >= nc * nc) return;
-    const int64_t col = t / nc, row = t % nc;      // column-major S
-    const int64_t n_cam = 15 * (int64_t)C;
-    double v = 0.0;
-    if (row >= nl || col >= nl) {
-        if (row == col) { rhs[row] = 0.0; gcopy[row] = 0.0; }
-    } else if (row < n_cam && col < n_cam) {
-        const int c = (int)(row / 15), a = (int)(row % 15), cb = (int)(col / 15), b = (int)(col % 15);
-        if (c == cb) {
-            const unsigned mask = cam_mask[c];
-            const bool fa = mask & (1u << a), fb = mask & (1u << b);
-            v = (fa && fb) ? U[(int64_t)c * 225 + a * 15 + b] : 0.0;
-            if (a == b) {
-                v = fa ? v + lambda * v : 0.0;
-                rhs[row] = fa ? -gc[row] : 0.0;
-                gcopy[row] = fa ? gc[row] : 0.0;
-            }
-        }
-    } else if (row >= n_cam && col >= n_cam) {
-        const int64_t jr = row - n_cam, jc = col - n_cam;
-        const int m = (int)(jr / 6), a = (int)(jr % 6), mb = (int)(jc / 6), b = (int)(jc % 6);
-        if (m == mb) {
-            const unsigned mask = pose_mask[m];
-            const bool fa = mask & (1u << a), fb = mask & (1u << b);
-            v = (fa && fb) ? V[(int64_t)m * 36 + a * 6 + b] : 0.0;
-            if (a == b) {
-                v = fa ? v + lambda * v : 0.0;
-                rhs[row] = fa ? -gp[jr] : 0.0;
-                gcopy[row] = fa ? gp[jr] : 0.0;
-            }
-        }
-    } else if (row >= n_cam) {   // pose row, camera column: W_s[a][j]
-        const int64_t jr = row - n_cam;
-        const int m = (int)(jr / 6), j = (int)(jr % 6), c = (int)(col / 15), a = (int)(col % 15);
-        const int32_t s = seg_of[(int64_t)c * M + m];
-        if (s >= 0 && (pose_mask[m] & (1u << j)) && (cam_mask[c] & (1u << a))) v = W[(int64_t)s * 90 + a * 6 + j];
-    }
-    Smat[t] = v;
 }
 
 // Z rows of the point elimination: for reduced row r (camera or pose unknown) and point k, z = x L_k^-T with x the 1 x 3
@@ -416,55 +332,12 @@ k_lm_point_elim_Z(int C, int M, int K, int64_t nc, int64_t nl, const double* __r
         double z[3] = {0.0, 0.0, 0.0};
         if (row_free) {
             const double* x = is_cam ? Xck + (((int64_t)blk * K + k) * 15 + a) * 3 : Ymk + (((int64_t)blk * K + k) * 6 + a) * 3;
-            const unsigned km = key_mask[k];
-            const double* Lk = L + (int64_t)k * 9;
-#pragma unroll
-            for (int i = 0; i < 3; ++i) {
-                double v = (km & (1u << i)) ? x[i] : 0.0;
-#pragma unroll
-                for (int q = 0; q < i; ++q) v -= Lk[i * 3 + q] * z[q];
-                z[i] = v / Lk[i * 3 + i];
-                dot = fma(z[i], y[3 * (int64_t)k + i], dot);
-            }
+            tri_row<3>(x, true, key_mask[k], L + (int64_t)k * 9, y, k, z, dot);
         }
 #pragma unroll
         for (int i = 0; i < 3; ++i) Z[(3 * (int64_t)k + i) * nc + r] = z[i];   // every entry is written: no memset
     }
     if (dot != 0.0) atomicAdd(rhs + r, -dot);
-}
-
-// delta_k = L_k^-T (y_k - Z_k^T delta_r), one warp per point; written behind the camera part of `dck`
-__global__ void __launch_bounds__(128)
-k_lm_point_back(int K, int64_t nc, const double* __restrict__ L, const double* __restrict__ y, const double* __restrict__ Z,
-                const double* __restrict__ delta_r, double* __restrict__ delta_k)
-{
-    const int k = (int)((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    if (k >= K) return;
-    double t[3] = {0.0, 0.0, 0.0};
-    const double* Zk = Z + 3 * (int64_t)k * nc;
-    for (int64_t r = lane; r < nc; r += 32) {
-        const double d = delta_r[r];
-#pragma unroll
-        for (int i = 0; i < 3; ++i) t[i] = fma(Zk[i * nc + r], d, t[i]);
-    }
-#pragma unroll
-    for (int i = 0; i < 3; ++i)
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) t[i] += __shfl_xor_sync(0xffffffffu, t[i], o);
-    if (lane != 0) return;
-    const double* Lk = L + (int64_t)k * 9;
-    double v[3];
-#pragma unroll
-    for (int i = 0; i < 3; ++i) v[i] = y[3 * (int64_t)k + i] - t[i];
-#pragma unroll
-    for (int i = 2; i >= 0; --i) {
-        double s = v[i];
-#pragma unroll
-        for (int q = i + 1; q < 3; ++q) s -= Lk[q * 3 + i] * v[q];
-        v[i] = s / Lk[i * 3 + i];
-    }
-#pragma unroll
-    for (int i = 0; i < 3; ++i) delta_k[3 * (int64_t)k + i] = v[i];
 }
 
 // rows whose diagonal is exactly zero after the reduction (fixed, or unobserved by every rank) -> identity
@@ -474,47 +347,53 @@ __global__ void k_lm_fix_diag(int64_t nc, double* __restrict__ Smat)
     if (a < nc && Smat[a * nc + a] == 0.0) Smat[a * nc + a] = 1.0;
 }
 
-// delta_p = L^-T (y - Z_m^T delta_c), one warp per pose: the six dot products t_i = Z[:, 6 m + i] . delta_c (Z is
-// column-major with nc contiguous rows per pose column, so the lanes stride over one column: coalesced) are formed here
-// instead of by a library GEMV over the whole of Z, then lane 0 runs the 6 x 6 back substitution.
+// delta_b = L_b^-T (y_b - Z_b^T delta_r), one warp per eliminated block: the B dot products t_i = Z[:, B slot(b) + i] .
+// delta_r (Z is column-major with nc contiguous rows per column, so the lanes stride over one column: coalesced) are
+// formed here instead of by a library GEMV over the whole of Z, then lane 0 runs the B x B back substitution.  delta_r is
+// the solution of the reduced system (all nc rows); delta_b the set's part of the parameter-string step.
+template <int B>
 __global__ void __launch_bounds__(128)
-k_lm_pose_back(int M, int64_t nc, const double* __restrict__ L, const double* __restrict__ y, const double* __restrict__ Z,
-               const int32_t* __restrict__ pose_slot, const double* __restrict__ delta_c, double* __restrict__ delta_p)
+k_lm_block_back(int n, int64_t nc, const double* __restrict__ L, const double* __restrict__ y, const double* __restrict__ Z,
+                const int32_t* __restrict__ slot, const double* __restrict__ delta_r, double* __restrict__ delta_b)
 {
     const int m = (int)((blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    if (m >= M) return;
-    double t[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-    const double* Zm = Z + (int64_t)(pose_slot ? pose_slot[m] : m) * 6 * nc;
-    for (int64_t a = lane; a < nc; a += 32) {
-        const double d = delta_c[a];
+    if (m >= n) return;
+    double t[B];
 #pragma unroll
-        for (int i = 0; i < 6; ++i) t[i] = fma(Zm[i * nc + a], d, t[i]);
+    for (int i = 0; i < B; ++i) t[i] = 0.0;
+    const double* Zm = Z + (int64_t)(slot ? slot[m] : m) * B * nc;
+    for (int64_t a = lane; a < nc; a += 32) {
+        const double d = delta_r[a];
+#pragma unroll
+        for (int i = 0; i < B; ++i) t[i] = fma(Zm[i * nc + a], d, t[i]);
     }
 #pragma unroll
-    for (int i = 0; i < 6; ++i)
+    for (int i = 0; i < B; ++i)
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) t[i] += __shfl_xor_sync(0xffffffffu, t[i], o);
     if (lane != 0) return;
-    const double* Lm = L + (int64_t)m * 36;
-    double v[6];
+    const double* Lm = L + (int64_t)m * (B * B);
+    double v[B];
 #pragma unroll
-    for (int i = 0; i < 6; ++i) v[i] = y[(int64_t)m * 6 + i] - t[i];
+    for (int i = 0; i < B; ++i) v[i] = y[(int64_t)m * B + i] - t[i];
 #pragma unroll
-    for (int i = 5; i >= 0; --i) {
+    for (int i = B - 1; i >= 0; --i) {
         double s = v[i];
 #pragma unroll
-        for (int k = i + 1; k < 6; ++k) s -= Lm[k * 6 + i] * v[k];
-        v[i] = s / Lm[i * 6 + i];
+        for (int k = i + 1; k < B; ++k) s -= Lm[k * B + i] * v[k];
+        v[i] = s / Lm[i * B + i];
     }
 #pragma unroll
-    for (int i = 0; i < 6; ++i) delta_p[(int64_t)m * 6 + i] = v[i];
+    for (int i = 0; i < B; ++i) delta_b[(int64_t)m * B + i] = v[i];
 }
 
-// delta (parameter-string layout): [intr | extr | pose (| point)] from delta_A (15 per camera, then 3 per key) and delta_p.
-// Also accumulates pred = sum delta (lambda D delta + b), |delta|^2, |x|^2 and |g|_inf of the LOCAL pose part
-// plus (rank 0 only for the replicated camera / point norms) the replicated part; D and b are this rank's partial sums.
+// delta (parameter-string layout): [intr | extr | pose (| point)] from the camera (15 per camera), pose and point parts of
+// the step, each read from the reduced solution or, for the eliminated set, from delta itself (written by
+// k_lm_block_back).  Also accumulates pred = sum delta (lambda D delta + b), |delta|^2, |x|^2 and |g|_inf of the LOCAL
+// pose part plus (rank 0 only for the replicated camera / point norms) the replicated part; D and b are this rank's
+// partial sums.
 __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const double* __restrict__ dc, const double* __restrict__ dp,
-                                    const double* __restrict__ U, const double* __restrict__ gc, const double* __restrict__ V,
+                                    const double* __restrict__ dk, const double* __restrict__ U, const double* __restrict__ gc, const double* __restrict__ V,
                                     const double* __restrict__ gp, const double* __restrict__ Pk, const double* __restrict__ gk,
                                     const uint16_t* __restrict__ cam_mask, const uint8_t* __restrict__ pose_mask,
                                     const uint8_t* __restrict__ key_mask, const double* __restrict__ params,
@@ -548,7 +427,7 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
             const int64_t j = t - n_cam - n_pose;
             const int k = (int)(j / 3), a = (int)(j % 3);
             f = key_mask[k] & (1u << a);
-            d = f ? dc[n_cam + j] : 0.0;
+            d = f ? dk[j] : 0.0;
             D = f ? Pk[(int64_t)k * 9 + a * 4] : 0.0;
             g = f ? gk[j] : 0.0;
             replicated = true;
@@ -585,13 +464,8 @@ __global__ void k_lm_assemble_delta(int C, int M, int K3, double lambda, const d
     }
 }
 
-__global__ void k_axpy_params(int64_t n, const double* __restrict__ delta, double* __restrict__ params)
-{
-    int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i < n) params[i] += delta[i];
-}
-
 // backup <- params, params += delta (the move to the trial point), and scal[4] = |g_cam|_inf in the same launch
+// (nc = 0, the dense fallback: the move alone)
 __global__ void k_lm_take_step(int64_t L, int64_t nc, const double* __restrict__ delta, double* __restrict__ params,
                                double* __restrict__ backup, const double* __restrict__ gcopy, double* __restrict__ scal)
 {
@@ -715,7 +589,6 @@ void lm_free(pcs_problem* p)
     if (w->ne_alt && w->ne_orig && p->ne == w->ne_alt) swap_normal_buffers(p, w);
     schur_plan_free(&w->plan);
     if (w->seg_of) cudaFree(w->seg_of);
-    if (w->dck) cudaFree(w->dck);
     double* ptrs[] = {w->L, w->y, w->Z, w->red, w->delta, w->backup, w->scal, w->Hd, w->rhs, w->Ldiag, w->ne_alt, w->cov_Xi};
     for (double* q : ptrs) if (q) cudaFree(q);
     if (w->info) cudaFree(w->info);
@@ -729,15 +602,47 @@ void lm_free(pcs_problem* p)
     p->lm_ws = nullptr;
 }
 
+// The LM path of the problem: the one its workspace was built for, else the one a workspace built now takes.  Template
+// chain: the poses are eliminated.  Self-calibration chain: poses AND points are block diagonal but coupled to each other,
+// so only one of them can go; the larger one does (3 K point unknowns against 6 M pose unknowns -- on the reference's
+// ccube fixture a reduced system of 162 instead of 1503 unknowns).  The point elimination is single-rank: its reduced
+// system contains the (rank-local) poses.  Without the (camera, key) / (pose, key) tables (p->Pk) the self-calibration
+// chain takes the dense fallback.  Switch for A/B runs and tests, read whenever a workspace is built:
+// PCS_LM_SELFCAL=dense forces the dense fallback of the self-calibration chain, PCS_LM_SELFCAL=poses its pose elimination.
+static LmPath lm_path(const pcs_problem* p)
+{
+    if (p->lm_ws) return ((const LmWorkspace*)p->lm_ws)->path;
+    if (p->chain == PCS_CHAIN_TEMPLATE) return {6, 0};
+    const char* env = std::getenv("PCS_LM_SELFCAL");
+    if (!p->Pk || (env && env[0] == 'd')) return {0, 0};
+    const bool points = p->world == 1 && 3 * (int64_t)p->K > 6 * (int64_t)p->M && !(env && env[0] == 'p');
+    return points ? LmPath{3, 6} : LmPath{6, 3};
+}
+
+// the block set B of the problem's current normal-equation outputs (B = 0: the empty set)
+static BlockSet block_set(const pcs_problem* p, const LmWorkspace* w, int B)
+{
+    BlockSet s;
+    s.B = B;
+    if (B == 6) {
+        s.n = p->M; s.off = 15 * (int64_t)p->C; s.blk = p->V; s.g = p->gp; s.mask = p->pose_mask; s.slot = w->plan.pose_slot;
+    } else if (B == 3) {
+        s.n = p->K; s.off = 15 * (int64_t)p->C + 6 * (int64_t)p->M; s.blk = p->Pk; s.g = p->gk; s.mask = p->key_mask;
+    }
+    return s;
+}
+
 static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w);
 
 // The workspace is published on the problem only after every allocation succeeded; a failure half-way (out of memory
 // for Z, n_free over the dense limit, ...) frees what was built, so that the next call starts from scratch instead of
-// launching on NULL buffers.
+// launching on NULL buffers.  It is laid out for the world size of the moment (the path, the all-reduce buffers):
+// pcs_set_allreduce frees it when the world size changes.
 static int lm_prepare(pcs_problem* p)
 {
     if (p->lm_ws) return PCS_OK;
     LmWorkspace* w = new LmWorkspace();
+    w->path = lm_path(p);
     p->lm_ws = w;
     const int rc = lm_prepare_impl(p, w);
     if (rc != PCS_OK) lm_free(p);
@@ -746,12 +651,9 @@ static int lm_prepare(pcs_problem* p)
 
 static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
 {
-    // Solver switches for A/B runs and tests, read whenever a workspace is built: PCS_LM_SELFCAL=dense forces the dense
-    // fallback of the self-calibration chain, PCS_LM_SELFCAL=poses its pose elimination, PCS_LM_SCHUR=dense the full
-    // iteration space (identity column order) of the pose elimination.
-    const char* env_selfcal = std::getenv("PCS_LM_SELFCAL");
+    // PCS_LM_SCHUR=dense (A/B runs and tests, read whenever a workspace is built): the full iteration space (identity
+    // column order) of the pose elimination
     const char* env_schur = std::getenv("PCS_LM_SCHUR");
-    const bool force_dense = env_selfcal && env_selfcal[0] == 'd', force_poses = env_selfcal && env_selfcal[0] == 'p';
     const bool dense_schur = env_schur && env_schur[0] == 'd';
     PCS_CUDA(cudaMalloc((void**)&w->delta, (size_t)p->L * 8));
     PCS_CUDA(cudaMalloc((void**)&w->backup, (size_t)p->L * 8));
@@ -762,37 +664,29 @@ static int lm_prepare_impl(pcs_problem* p, LmWorkspace* w)
     PCS_CUDA(cudaMemsetAsync(w->delta, 0, (size_t)p->L * 8, p->stream));
     PCS_CUDA(cudaEventCreate(&w->ev0));
     PCS_CUDA(cudaEventCreate(&w->ev1));
-    if (p->chain == PCS_CHAIN_TEMPLATE || (p->Pk && !force_dense)) {
-        // Which block set is eliminated.  Template chain: the poses.  Self-calibration chain: poses AND points are block
-        // diagonal but coupled to each other, so only one of them can go; the larger one does (3 K point unknowns against
-        // 6 M pose unknowns).  The point elimination is single-rank: its reduced system contains the (rank-local) poses.
-        w->pts_elim = p->chain == PCS_CHAIN_SELFCAL && p->world == 1 && 3 * (int64_t)p->K > 6 * (int64_t)p->M && !force_poses;
-        if (w->pts_elim) {
-            w->nl = 15 * (int64_t)p->C + 6 * (int64_t)p->M;       // cameras + poses
-            w->np = 3 * (int64_t)p->K;                            // eliminated: point coordinates
-        } else {
-            w->nl = 15 * (int64_t)p->C + (p->chain == PCS_CHAIN_SELFCAL ? 3 * (int64_t)p->K : 0);   // cameras (+ target points)
-            w->np = 6 * (int64_t)p->M;
-        }
+    if (w->path.elim_B) {
+        const BlockSet e = block_set(p, w, w->path.elim_B), r = block_set(p, w, w->path.red_B);
+        w->nl = 15 * (int64_t)p->C + (int64_t)r.B * r.n;   // cameras (+ the second set)
+        w->np = (int64_t)e.B * e.n;                        // eliminated unknowns
         w->nc = (w->nl + 31) / 32 * 32;
-        PCS_CUDA(cudaMalloc((void**)&w->L, (size_t)(w->pts_elim ? (int64_t)p->K * 9 : (int64_t)p->M * 36) * 8));
+        PCS_CUDA(cudaMalloc((void**)&w->L, (size_t)(w->np * e.B) * 8));
         PCS_CUDA(cudaMalloc((void**)&w->y, (size_t)w->np * 8));
         PCS_CUDA(cudaMalloc((void**)&w->Z, (size_t)(w->nc * w->np) * 8));
         PCS_CUDA(cudaMemsetAsync(w->Z, 0, (size_t)(w->nc * w->np) * 8, p->stream));  // sparsity pattern is static
-        if (w->pts_elim) {
+        if (r.B == 6) {
             PCS_CUDA(cudaMalloc((void**)&w->seg_of, (size_t)p->C * p->M * sizeof(int32_t)));
             PCS_CUDA(cudaMemsetAsync(w->seg_of, 0xff, (size_t)p->C * p->M * sizeof(int32_t), p->stream));
             if (p->n_seg) k_seg_of<<<grid_for(p->n_seg, 256), 256, 0, p->stream>>>(p->n_seg, p->M, p->seg_cam, p->seg_pose, w->seg_of);
             PCS_CUDA(cudaGetLastError());
-            PCS_CUDA(cudaMalloc((void**)&w->dck, (size_t)(15 * (int64_t)p->C + 3 * (int64_t)p->K) * 8));
         }
         // block-sparse pose elimination
-        if (!w->pts_elim && !dense_schur) PCS_TRY(schur_plan_build(p, w->nc, w->nl, &w->plan));
+        if (e.B == 6 && !dense_schur) PCS_TRY(schur_plan_build(p, w->nc, w->nl, &w->plan));
         w->red_doubles = w->nc * w->nc + 2 * w->nc + 1;
         PCS_CUDA(cudaMalloc((void**)&w->red, (size_t)w->red_doubles * 8));
         PCS_TRY(chol_prepare(p->device, w->nc, &w->Ldiag, &w->bar, &w->chol_grid));
         PCS_CUDA(cudaMalloc((void**)&w->ne_alt, (size_t)p->ne_doubles * 8));
         w->ne_orig = p->ne;
+        PCS_CUDA(cudaMalloc((void**)&w->comb, (size_t)(5 + p->world) * 8));
     } else {
         const int64_t n = p->n_free;
         PCS_REQUIRE(n > 0 && n <= 32768, "dense LM path needs 0 < n_free <= 32768");
@@ -816,39 +710,34 @@ static int eval_normal(pcs_problem* p)
 
 // The reduced system at damping lambda, built in w->red and ready for the factorisation: S (lower triangle; fixed and
 // unobserved unknowns are identity rows), rhs = -g_red - Z y, the gradient copy and the cost; w->L / w->y hold the
-// eliminated blocks' Cholesky factors and L_b^-1 (-g_b), w->Z the coupling W L_b^-T.  Multi-rank: S | rhs | g | cost are
+// eliminated blocks' Cholesky factors and L_b^-1 (-g_b), w->Z the coupling L_b^-T.  Multi-rank: S | rhs | g | cost are
 // all-reduced here.  The first half of every LM step, and what pcs_covariance factors at lambda = 0.
 static int build_reduced(pcs_problem* p, LmWorkspace* w, double lambda)
 {
     cudaStream_t st = p->stream;
     const int64_t nc = w->nc, np = w->np;
+    const BlockSet e = block_set(p, w, w->path.elim_B), r = block_set(p, w, w->path.red_B);
     double* Smat = w->red;
     double* rhs = w->red + nc * nc;
     double* gcopy = rhs + nc;
     double* cost_r = gcopy + nc;
-    if (w->pts_elim) {   // self-calibration chain, points eliminated
-        k_lm_init_reduced_cp<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, p->M, nc, w->nl, lambda, p->U, p->gc, p->V, p->gp, p->W,
-                                                                                         w->seg_of, p->cost, p->cam_mask, p->pose_mask, Smat, rhs,
-                                                                                         gcopy, cost_r, w->scal, w->info);
-        k_lm_point_factor<<<grid_for(p->K, 128), 128, 0, st>>>(p->K, lambda, p->Pk, p->gk, p->key_mask, w->L, w->y, w->scal);
+    const auto init = r.B == 6 ? k_lm_init_reduced<6> : k_lm_init_reduced<3>;
+    init<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, r.n, nc, w->nl, lambda, p->U, p->gc, p->cost, p->cam_mask,
+                                                                      r.blk, r.g, r.mask, p->Xck, p->W, w->seg_of, Smat, rhs, gcopy,
+                                                                      cost_r, w->scal, w->info);
+    const auto factor = e.B == 6 ? k_lm_block_factor<6> : k_lm_block_factor<3>;
+    factor<<<grid_for(e.n, 128), 128, 0, st>>>(e.n, lambda, e.blk, e.g, e.mask, w->L, w->y, w->scal);
+    if (e.B == 3) {
         k_lm_point_elim_Z<<<dim3(grid_for(nc, 128), (p->K + PT_CHUNK - 1) / PT_CHUNK), 128, 0, st>>>(p->C, p->M, p->K, nc, w->nl, p->Xck, p->Ymk, w->L,
                                                                                                   w->y, p->cam_mask, p->pose_mask, p->key_mask, w->Z, rhs);
-        PCS_CUDA(cudaGetLastError());
-        PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, nullptr));
-        k_lm_fix_diag<<<grid_for(nc, 256), 256, 0, st>>>(nc, Smat);
-        return PCS_OK;
+    } else {
+        if (p->n_seg)
+            k_lm_segment_Z<<<grid_for(p->n_seg * 15, 256), 256, 0, st>>>(p->n_seg, nc, p->seg_cam, p->seg_pose, p->W, w->L, w->y,
+                                                                         p->cam_mask, p->pose_mask, e.slot, w->Z, rhs);
+        if (r.B == 3)
+            k_lm_point_Z<<<grid_for((int64_t)p->M * p->K * 3, 256), 256, 0, st>>>(p->M, p->K, nc, 15 * (int64_t)p->C, p->Ymk, w->L, w->y,
+                                                                                 p->pose_mask, p->key_mask, e.slot, w->Z, rhs);
     }
-    const bool selfcal = p->chain == PCS_CHAIN_SELFCAL;
-    k_lm_init_reduced<<<grid_for(std::max<int64_t>(nc * nc, 9), 256), 256, 0, st>>>(p->C, p->K, nc, w->nl, lambda, p->U, p->gc, p->cost, p->cam_mask,
-                                                                                  p->Pk, p->gk, p->Xck, p->key_mask,
-                                                                                  Smat, rhs, gcopy, cost_r, w->scal, w->info);
-    k_lm_pose_factor<<<grid_for(p->M, 128), 128, 0, st>>>(p->M, lambda, p->V, p->gp, p->pose_mask, w->L, w->y, w->scal);
-    if (p->n_seg)
-        k_lm_segment_Z<<<grid_for(p->n_seg * 15, 256), 256, 0, st>>>(p->n_seg, nc, p->seg_cam, p->seg_pose, p->W, w->L, w->y,
-                                                                     p->cam_mask, p->pose_mask, w->plan.pose_slot, w->Z, rhs);
-    if (selfcal)
-        k_lm_point_Z<<<grid_for((int64_t)p->M * p->K * 3, 256), 256, 0, st>>>(p->M, p->K, nc, 15 * (int64_t)p->C, p->Ymk, w->L, w->y,
-                                                                             p->pose_mask, p->key_mask, w->plan.pose_slot, w->Z, rhs);
     PCS_CUDA(cudaGetLastError());
     PCS_TRY(launch_schur_syrk(st, p->sm_count, nc, np, w->Z, Smat, &w->plan));
     if (p->allreduce) {
@@ -867,45 +756,29 @@ static int chol_solve(pcs_problem* p, LmWorkspace* w, int64_t n, double* A, int6
     return launch_chol_solve(p->stream, w->chol_grid, n, A, ld, rhs, w->Ldiag, w->bar, &w->bar_base, w->info);
 }
 
-// Self-calibration chain, points eliminated (w->pts_elim): same contract as solve_template below.
-static int solve_points_eliminated(pcs_problem* p, LmWorkspace* w, double lambda)
+// One damped solve of the block path at the current linearisation, enqueued without synchronising.  Afterwards w->delta
+// holds the step (parameter-string layout), w->scal = {pred, |dx|^2, |x|^2, |g_pose|_inf, |g_cam|_inf, flag, trial cost, -},
+// w->info the factorisation status and cost_r (inside w->red) the all-reduced r.r of the linearisation point.
+static int solve_step(pcs_problem* p, LmWorkspace* w, double lambda)
 {
     cudaStream_t st = p->stream;
     const int64_t nc = w->nc, n_cam = 15 * (int64_t)p->C;
     double* rhs = w->red + nc * nc;
     PCS_TRY(build_reduced(p, w, lambda));
     PCS_TRY(chol_solve(p, w, nc, w->red, nc, rhs));
-    p->n_launches += 7;
-    // rhs now holds [delta_c | delta_m]; the points follow from the back substitution
-    PCS_CUDA(cudaMemcpyAsync(w->dck, rhs, (size_t)n_cam * 8, cudaMemcpyDeviceToDevice, st));
-    k_lm_point_back<<<grid_for((int64_t)p->K * 32, 128), 128, 0, st>>>(p->K, nc, w->L, w->y, w->Z, rhs, w->dck + n_cam);
-    const int K3 = 3 * p->K;
+    const BlockSet e = block_set(p, w, w->path.elim_B);
+    p->n_launches += e.B == 6 ? 8 : 7;
+    // rhs now holds the reduced part of the step (cameras, then the second set); the eliminated set's part is written in
+    // place into the parameter-string delta
+    double* de = w->delta + e.off;
+    const auto back = e.B == 6 ? k_lm_block_back<6> : k_lm_block_back<3>;
+    back<<<grid_for((int64_t)e.n * 32, 128), 128, 0, st>>>(e.n, nc, w->L, w->y, w->Z, e.slot, rhs, de);
+    const double* dp = e.B == 6 ? de : rhs + n_cam;
+    const double* dk = e.B == 3 ? de : rhs + n_cam;
+    const int K3 = p->chain == PCS_CHAIN_SELFCAL ? 3 * p->K : 0;
     k_lm_assemble_delta<<<grid_for(n_cam + 6 * (int64_t)p->M + K3, 128), 128, 0, st>>>(
-        p->C, p->M, K3, lambda, w->dck, rhs + n_cam, p->U, p->gc, p->V, p->gp, p->Pk, p->gk, p->cam_mask, p->pose_mask, p->key_mask, p->params,
-        w->delta, w->scal, 1, 1);
-    PCS_CUDA(cudaGetLastError());
-    return PCS_OK;
-}
-
-// One damped solve at the current linearisation, enqueued without synchronising.  Afterwards w->delta holds the step
-// (parameter-string layout), w->scal = {pred, |dx|^2, |x|^2, |g_pose|_inf, |g_cam|_inf, flag, trial cost, -},
-// w->info the factorisation status and cost_r (inside w->red) the all-reduced r.r of the linearisation point.
-static int solve_template(pcs_problem* p, LmWorkspace* w, double lambda)
-{
-    cudaStream_t st = p->stream;
-    const int64_t nc = w->nc;
-    double* rhs = w->red + nc * nc;
-    const bool selfcal = p->chain == PCS_CHAIN_SELFCAL;
-    PCS_TRY(build_reduced(p, w, lambda));
-    PCS_TRY(chol_solve(p, w, nc, w->red, nc, rhs));
-    p->n_launches += 8;
-    // rhs now holds delta_c
-    double* dp = w->delta + 15 * (int64_t)p->C;  // pose part of the parameter-string delta is written in place
-    k_lm_pose_back<<<grid_for((int64_t)p->M * 32, 128), 128, 0, st>>>(p->M, nc, w->L, w->y, w->Z, w->plan.pose_slot, rhs, dp);
-    const int K3 = selfcal ? 3 * p->K : 0;
-    k_lm_assemble_delta<<<grid_for(15 * (int64_t)p->C + 6 * (int64_t)p->M + K3, 128), 128, 0, st>>>(
-        p->C, p->M, K3, lambda, rhs, dp, p->U, p->gc, p->V, p->gp, p->Pk, p->gk, p->cam_mask, p->pose_mask, p->key_mask, p->params,
-        w->delta, w->scal, p->rank == 0, 0);
+        p->C, p->M, K3, lambda, rhs, dp, dk, p->U, p->gc, p->V, p->gp, p->Pk, p->gk, p->cam_mask, p->pose_mask, p->key_mask,
+        p->params, w->delta, w->scal, p->rank == 0, e.B == 3);
     PCS_CUDA(cudaGetLastError());
     return PCS_OK;   // multi-rank: pred, |dx|^2, |x|^2 and the pose gradient norm are still rank-local here (k_lm_pack_scalars)
 }
@@ -936,17 +809,13 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
     PCS_CUDA(cudaSetDevice(p->device));
     pcs_lm_options o;
     if (opts_in) o = *opts_in; else pcs_lm_default_options(&o);
-    if (p->chain == PCS_CHAIN_SELFCAL && p->world > 1 && !p->Pk) {
+    if (p->world > 1 && lm_path(p).elim_B == 0) {
         // the dense self-calibration fallback is not combined across ranks: refuse instead of letting the replicated
         // camera / point parameters diverge silently
         set_error("pcs_lm_solve: the dense self-calibration fallback is single-rank");
         return PCS_ERR_UNSUPPORTED;
     }
     PCS_TRY(lm_prepare(p));
-    if (((LmWorkspace*)p->lm_ws)->pts_elim && p->world > 1) {   // the all-reduce hook was installed after the workspace was built
-        lm_free(p);
-        PCS_TRY(lm_prepare(p));
-    }
     LmWorkspace* w = (LmWorkspace*)p->lm_ws;
     cudaStream_t st = p->stream;
     cudaEvent_t ev0 = w->ev0, ev1 = w->ev1;
@@ -957,14 +826,7 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
         PCS_CUDA(cudaMemcpyAsync(p->x, p->h_pin, (size_t)p->n_free * 8, cudaMemcpyHostToDevice, st));
         PCS_TRY(launch_scatter_x(p, p->x));
     }
-    if (w->comb_cap < 5 + p->world) {   // the world size may have been set after the workspace was created
-        if (w->comb) cudaFree(w->comb);
-        w->comb = nullptr;
-        w->comb_cap = 0;
-        PCS_CUDA(cudaMalloc((void**)&w->comb, (size_t)(5 + p->world) * 8));
-        w->comb_cap = 5 + p->world;
-    }
-    const bool tmpl = w->nc > 0;   // block path (both chains); false: dense self-calibration fallback
+    const bool block = w->path.elim_B != 0;   // block path (both chains); false: dense self-calibration fallback
     const int64_t n = p->n_free;
     int n_normal = 0, n_cost = 0, status = 0, it = 0;
     double lambda = o.lambda0, nu = 2.0;
@@ -973,7 +835,7 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
 
     auto eval_lin = [&]() -> int {  // normal equations at p->params; returns r.r in `cost`
         ++n_normal;
-        if (tmpl) return eval_normal(p);
+        if (block) return eval_normal(p);
         return pcs_normal_dense_dev_internal(p);
     };
     int rc = eval_lin();
@@ -982,12 +844,12 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
         ++it;
         double ginf_cam = 0.0, cost_lin = 0.0, cost_new = 0.0;
         int h_info = 0;
-        if (tmpl) {
-            // Template chain: the damped solve, the step and the evaluation of the TRIAL point with the full
+        if (block) {
+            // Block path: the damped solve, the step and the evaluation of the TRIAL point with the full
             // normal-equation kernel (into the second output set) are enqueued back to back and read with ONE
             // synchronisation per iteration.  An accepted step already has its linearisation; a rejected one only
             // costs the difference between the full kernel and a residual-only pass.
-            rc = w->pts_elim ? solve_points_eliminated(p, w, lambda) : solve_template(p, w, lambda);
+            rc = solve_step(p, w, lambda);
             if (rc != PCS_OK) break;
             double* gcopy = w->red + w->nc * w->nc + w->nc;
             k_lm_take_step<<<grid_for(std::max<int64_t>(p->L, w->nc), 256), 256, 0, st>>>(p->L, w->nc, w->delta, p->params, w->backup,
@@ -1027,9 +889,9 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
             PCS_CUDA(cudaStreamSynchronize(st));
             rc = chol_status(h_info);
         }
-        // the template chain has already moved to the trial point: undo = old parameters + old output set
+        // the block path has already moved to the trial point: undo = old parameters + old output set
         auto undo_trial = [&]() -> int {
-            if (!tmpl) return PCS_OK;
+            if (!block) return PCS_OK;
             PCS_CUDA(cudaMemcpyAsync(p->params, w->backup, (size_t)p->L * 8, cudaMemcpyDeviceToDevice, st));
             swap_normal_buffers(p, w);
             --n_normal;   // the speculative evaluation is not a linearisation that was used
@@ -1048,10 +910,9 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
         if (ginf < o.gtol) { status = 1; rc = undo_trial(); break; }
         const double pred = h_scal[0], dx = std::sqrt(h_scal[1]), xn = std::sqrt(h_scal[2]);
         if (dx < o.xtol * (o.xtol + xn)) { status = 3; rc = undo_trial(); break; }
-        if (!tmpl) {
+        if (!block) {
             // trial point, residual-only pass
-            PCS_CUDA(cudaMemcpyAsync(w->backup, p->params, (size_t)p->L * 8, cudaMemcpyDeviceToDevice, st));
-            k_axpy_params<<<grid_for(p->L, 256), 256, 0, st>>>(p->L, w->delta, p->params);
+            k_lm_take_step<<<grid_for(p->L, 256), 256, 0, st>>>(p->L, 0, w->delta, p->params, w->backup, nullptr, w->scal);
             PCS_TRY(launch_prepare(p));
             PCS_TRY(launch_cost_only(p, w->scal + 6));
             ++n_cost;
@@ -1074,20 +935,20 @@ static int lm_solve_impl(pcs_problem* p, const double* x0, const pcs_lm_options*
             const double f = 1.0 - std::pow(2.0 * rho - 1.0, 3.0);
             lambda = std::max(o.lambda_min, lambda * std::max(1.0 / 3.0, f));
             nu = 2.0;
-            if (!tmpl) {
+            if (!block) {
                 rc = eval_lin();
                 if (rc != PCS_OK) break;
             }
             if (rel < o.ftol) { status = 2; break; }
         } else {
-            if (tmpl) rc = undo_trial();
+            if (block) rc = undo_trial();
             else PCS_CUDA(cudaMemcpyAsync(p->params, w->backup, (size_t)p->L * 8, cudaMemcpyDeviceToDevice, st));
             lambda = std::min(o.lambda_max, lambda * nu);
             nu *= 2.0;
             if (lambda >= o.lambda_max) { status = -1; break; }
         }
     }
-    if (tmpl && p->ne != w->ne_orig) {   // callers hold pointers into the original output set (pcs_device_pointers)
+    if (block && p->ne != w->ne_orig) {   // callers hold pointers into the original output set (pcs_device_pointers)
         PCS_CUDA(cudaMemcpyAsync(w->ne_orig, p->ne, (size_t)p->ne_doubles * 8, cudaMemcpyDeviceToDevice, st));
         swap_normal_buffers(p, w);
     }
@@ -1127,16 +988,12 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
         set_error("pcs_covariance: the covariance is single-rank (an all-reduce hook is installed)");
         return PCS_ERR_UNSUPPORTED;
     }
-    if (p->chain == PCS_CHAIN_SELFCAL && !p->Pk) {
+    if (lm_path(p).elim_B == 0) {
         set_error("pcs_covariance: the dense self-calibration fallback has no block path to factor");
         return PCS_ERR_UNSUPPORTED;
     }
     PCS_TRY(lm_prepare(p));
     LmWorkspace* w = (LmWorkspace*)p->lm_ws;
-    if (w->nc == 0) {   // PCS_LM_SELFCAL=dense
-        set_error("pcs_covariance: the dense self-calibration fallback has no block path to factor");
-        return PCS_ERR_UNSUPPORTED;
-    }
     cudaStream_t st = p->stream;
     const int64_t nc = w->nc, np = w->np, n_cam = 15 * (int64_t)p->C;
     if (!w->cov_Xi) PCS_CUDA(cudaMalloc((void**)&w->cov_Xi, (size_t)(nc * nc) * 8));
@@ -1159,15 +1016,13 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
     // X = L^-1 [I | Z] in place (Z's columns become X_b), then Sigma_red = X_I^T X_I into S (negated), Sigma_bb over L_b
     PCS_TRY(cov_forward_substitution(st, nc, Smat, w->Ldiag, w->cov_Xi, w->Z, np));
     PCS_TRY(cov_reduced_inverse(st, p->sm_count, nc, w->cov_Xi, Smat));
-    const int elim_B = w->pts_elim ? 3 : 6;
-    const int n_elim = w->pts_elim ? p->K : p->M;
-    PCS_TRY(cov_block_marginals(st, n_elim, elim_B, nc, w->Z, w->pts_elim ? nullptr : w->plan.pose_slot, w->L));
+    const BlockSet e = block_set(p, w, w->path.elim_B);
+    PCS_TRY(cov_block_marginals(st, e.n, e.B, nc, w->Z, e.slot, w->L));
     // copy-out layout in the (now free) X_I buffer: cam [15 C][15 C], then the reduced set's pose or point blocks
-    const int red_B = w->pts_elim ? 6 : (p->chain == PCS_CHAIN_SELFCAL ? 3 : 0);
     double* out_cam = w->cov_Xi;
     double* out_red = w->cov_Xi + n_cam * n_cam;
     double* n_obs = w->scal + 7;   // cleared by the reduced-system build
-    PCS_TRY(cov_assemble(st, p, nc, red_B, elim_B, Smat, w->L, out_cam, out_red, n_obs));
+    PCS_TRY(cov_assemble(st, p, nc, w->path.red_B, e.B, Smat, w->L, out_cam, out_red, n_obs));
     // the LM path clears Z once and relies on its static zero pattern
     PCS_CUDA(cudaMemsetAsync(w->Z, 0, (size_t)(nc * np) * 8, st));
     double* h = w->h_read;
@@ -1186,8 +1041,8 @@ static int covariance_impl(pcs_problem* p, const double* x, double* cam, double*
     if (dof) *dof = d;
     if (s2) *s2 = d > 0 ? h[9] / (double)d : std::nan("");
     if (cam) PCS_CUDA(cudaMemcpyAsync(cam, out_cam, (size_t)(n_cam * n_cam) * 8, cudaMemcpyDeviceToHost, st));
-    double* pose_src = w->pts_elim ? out_red : (double*)w->L;
-    double* point_src = w->pts_elim ? (double*)w->L : out_red;
+    double* pose_src = e.B == 6 ? w->L : out_red;
+    double* point_src = e.B == 3 ? w->L : out_red;
     if (pose && p->M) PCS_CUDA(cudaMemcpyAsync(pose, pose_src, (size_t)p->M * 36 * 8, cudaMemcpyDeviceToHost, st));
     if (point && p->chain == PCS_CHAIN_SELFCAL && p->K)
         PCS_CUDA(cudaMemcpyAsync(point, point_src, (size_t)p->K * 9 * 8, cudaMemcpyDeviceToHost, st));

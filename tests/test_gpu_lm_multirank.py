@@ -176,7 +176,7 @@ def test_two_ranks_self_calibration_chain():
                 with BundleProblem(1, c_s, p_s, k_s, uv_s, Cn, ranges[r][1] - ranges[r][0], Kn, unfixed=unf) as p:
                     p.set_param_string(par)
                     # builds the solver workspace while the problem is still single-rank (it then plans to eliminate the
-                    # points); the hook installed afterwards must make the solve rebuild it for the pose elimination
+                    # points); installing the hook for two ranks frees it, and the solve rebuilds it for the pose elimination
                     assert p.lm_schur_fraction() == 1.0
                     p.set_allreduce(hs.hook(r), r, 2)
                     _, st = p.lm_solve(par[unf], max_iter=iters, ftol=0.0, xtol=0.0, gtol=0.0)
@@ -203,3 +203,17 @@ def test_two_ranks_self_calibration_chain():
         assert st0["iterations"] == st1["iterations"] == st["iterations"]
         assert abs(st0["cost_final"] - st["cost_final"]) <= 1e-9 * st["cost_final"], (st0, st)
         assert np.max(np.abs(full - ref) / np.maximum(1.0, np.abs(ref))) <= 1e-8
+
+
+def test_forced_dense_fallback_refuses_two_ranks():
+    """The dense self-calibration fallback does not combine the ranks' normal equations, so a solve on it with world_size
+    > 1 is refused -- also when PCS_LM_SELFCAL=dense forces it on a problem that has the block path."""
+    from pycamset_b200 import _lib as L
+    from tests import lm_reference as R
+    from tests.helpers import solver_env
+    fx = R.FIXTURES["ring5_fixedcam_selfcal"]()
+    with solver_env(PCS_LM_SELFCAL="dense"), fx.problem() as p:
+        p.set_allreduce(lambda ptr, n, op, stream: None, 0, 2)
+        with pytest.raises(L.PcsError) as e:
+            p.lm_solve(fx.x0, max_iter=1)
+        assert e.value.code == L.PCS_ERR_UNSUPPORTED
